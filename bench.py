@@ -16,6 +16,11 @@ Prints ONE JSON line (rank 0).
 
 (the other configs of BASELINE.json as one-line measurements of the same shape; the default is configs[1], the
 configuration the headline metric is quoted on).
+
+    python bench.py ... --dump-outputs DIR        # also write what the last timed step computed as DIR/<name>.npy
+
+The inputs depend on the arguments only (seeded mazes and actions), so the dumps of two builds run with the same
+arguments can be compared array for array.
 """
 from __future__ import annotations
 
@@ -38,6 +43,7 @@ UNIT = "env-steps/s"
 SHAPE = (81, 81)
 NUM_MAZES = 1000
 ALGO_BYTES_PER_STEP = 58   # SURVEY.md section 8(d): action 1 + state 16 + tables 7 + outputs 34
+DUMP_BYTES = 64 * 10**6
 
 
 def workload_name(envs_per_gpu):
@@ -289,6 +295,37 @@ def measure_extras(mb, torch, device):
     return out
 
 
+def env_step_outputs(env):
+    """The arrays MazeVectorEnv.step() returned for its last step: obs['agent'], obs['target'], obs['best dir'], reward,
+    terminated, truncated (they alias these output buffers of the batch)."""
+    b = env.batch
+    return {"agent": b.agent, "target": b.target, "best_dir": b.best_dir, "reward": b.reward,
+            "terminated": b.terminated, "truncated": b.truncated}
+
+
+def dump_outputs(path, arrays, seed=0):
+    """Write device arrays that share their first dimension (one row per env) as path/<name>.npy: float64 arrays as
+    float64, all others as float32 (exact for the coordinates, flags and float32 values written here).  When the rows
+    of all arrays would take more than DUMP_BYTES, the same fixed, seeded sample of rows is written from every array,
+    and the sampled row indices as rows.npy."""
+    import numpy as np
+    import torch
+    n = next(iter(arrays.values())).shape[0]
+    row_bytes = sum((8 if a.dtype == torch.float64 else 4) * (a.numel() // max(1, n)) for a in arrays.values())
+    budget = DUMP_BYTES - 128 * (len(arrays) + 1)      # .npy headers
+    rows = None
+    if n * row_bytes > budget:
+        rows = np.sort(np.random.default_rng(seed).choice(n, budget // (row_bytes + 8), replace=False))
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        if rows is not None:
+            a = a[torch.from_numpy(rows).to(a.device)]
+        a = a.double() if a.dtype == torch.float64 else a.float()
+        np.save(os.path.join(path, name + ".npy"), a.cpu().numpy())
+    if rows is not None:
+        np.save(os.path.join(path, "rows.npy"), rows.astype(np.float64))
+
+
 def pattern_summary(step_us, B):
     """Where the step kernel stands against the measured rate of its own access pattern (DESIGN.md section 4.1)."""
     p = pattern_peak()
@@ -372,6 +409,8 @@ def run_ours(args, rank, local_rank, world):
     e1.record()
     torch.cuda.synchronize()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, env_step_outputs(env))
     ms = max_over_ranks(evs[0].elapsed_time(e1))
     per_launch_us = sorted(evs[i].elapsed_time(evs[i + 1]) * 1e3 for i in range(n_ev))
     median_launch_us = per_launch_us[len(per_launch_us) // 2]
@@ -586,6 +625,8 @@ def run_toroidal_regen(args, rank, local_rank, world):
     args_w, args.warmup = args.warmup, 0
     ms = _timed_loop(torch, step, args, barrier, max_over_ranks)
     args.warmup = args_w
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, env_step_outputs(env))
     s1 = env.episode_statistics(reduce=world > 1)
     clocks = sampler.stop()
     if rank != 0:
@@ -635,6 +676,8 @@ def run_curriculum_dq(args, rank, local_rank, world):
     sampler = ClockSampler(local_rank)
     sampler.start()
     ms = _timed_loop(torch, step, args, barrier, max_over_ranks)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, env_step_outputs(env))
     clocks = sampler.stop()
     agent.core.check_overflow()
     stats = env.episode_statistics(reduce=world > 1)
@@ -672,6 +715,8 @@ def run_ddqn(args, rank, local_rank, world):
     args_w, args.warmup = args.warmup, 0
     ms = _timed_loop(torch, lambda: loop.iterate(time_allreduce=True), args, barrier, max_over_ranks)
     args.warmup = args_w
+    if args.dump_outputs and rank == 0:      # the env step plus the policy's Q values that chose its actions
+        dump_outputs(args.dump_outputs, dict(env_step_outputs(loop.env), q=loop.q))
     clocks = sampler.stop()
     ar_ms = sum(a.elapsed_time(b) for a, b in loop.ar_events)
     # the dominant kernel inside the step, measured live: maze_dqn_backward records a CUDA event after every launch while the
@@ -752,8 +797,8 @@ class JsonOnlyStdout:
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
-    ap.add_argument("--warmup", type=int, default=500)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: 2000 for configs1, 200 for the other workloads)")
+    ap.add_argument("--warmup", type=int, default=None, help="warm-up steps (default: 500 for configs1, 20 for the other workloads)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--envs-per-gpu", type=int, default=None)
     ap.add_argument("--workload", default="configs1", choices=["configs1", "toroidal-regen", "curriculum-dq", "ddqn"])
@@ -763,12 +808,20 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (rank 0's envs) as DIR/<name>.npy, at most 64 MB")
     args = ap.parse_args()
     args.envs_per_gpu_set = args.envs_per_gpu is not None
     if args.envs_per_gpu is None:
         args.envs_per_gpu = 4096 * NUM_MAZES
-    if args.workload != "configs1" and args.steps == 2000 and args.warmup == 500:   # the defaults are sized for 90 us steps
-        args.steps, args.warmup = 200, 20
+    if args.steps is None:      # configs1 steps take about 90 us, the other workloads' several times that
+        args.steps = 2000 if args.workload == "configs1" else 200
+    if args.warmup is None:
+        args.warmup = 500 if args.workload == "configs1" else 20
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -1,12 +1,12 @@
 #!/usr/bin/env python
-"""Copy the UNMODIFIED reference into baseline/_ref/ (git-ignored, travels to the GPU box with the snapshot).
+"""Copy the UNMODIFIED reference into baseline/_ref/ (git-ignored).
 
-    python tools/install_reference.py        # build container only: needs /root/reference
+    MAZE_REFERENCE_ROOT=<checkout of the reference> python tools/install_reference.py
 
 The reference has no setup.py / pyproject.toml, so there is nothing to pip-install (DESIGN.md section 5); a plain
-copy of its Python tree is the install.  baseline/_ref is test / bench infrastructure: tests/test_gpu_ref_consumer.py
-runs the reference's own agents/q_agent.py and lib/trainers/off_policy_trainer.py from it against this repo's env
-classes.  Nothing under maze-solving-agent-gymnasium_b200/ reads it, and none of it is committed.
+copy of its Python tree is the install.  baseline/_ref is bench infrastructure: where it is present,
+`bench.py --impl reference` times the reference's own SimpleMazeEnv instead of the oracle's port of it.  Nothing under
+maze-solving-agent-gymnasium_b200/ reads it, and none of it is committed.
 """
 from __future__ import annotations
 
