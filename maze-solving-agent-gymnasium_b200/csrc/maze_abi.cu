@@ -1,7 +1,6 @@
 // Context management and host-side helpers of the C ABI.
 #include <cmath>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <new>
 #include "maze_common.cuh"
@@ -83,25 +82,6 @@ extern "C" int maze_ctx_create(maze_ctx** out, int device) {
         cudaFree(ctx->d_counter);
         delete ctx;
         return rc;
-    }
-    ctx->step_ept = 2;
-    if (const char* v = getenv("MAZE_STEP_EPT")) ctx->step_ept = atoi(v);
-    if (const char* v = getenv("MAZE_L2_PERSIST_MB")) {   // experiment: L2 set-aside for evict_last / persisting lines
-        int maxp = 0;
-        cudaDeviceGetAttribute(&maxp, cudaDevAttrMaxPersistingL2CacheSize, device);
-        size_t want = (size_t)atoi(v) << 20, before = 0, after = 0;
-        if (want > (size_t)maxp) want = (size_t)maxp;
-        cudaDeviceGetLimit(&before, cudaLimitPersistingL2CacheSize);
-        cudaError_t le = cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want);
-        cudaDeviceGetLimit(&after, cudaLimitPersistingL2CacheSize);
-        fprintf(stderr, "[maze_b200] persisting L2 %zu -> %zu bytes (max %d, rc %d)\n", before, after, maxp, (int)le);
-    }
-    if (const char* v = getenv("MAZE_L2_FETCH")) {
-        size_t before = 0, after = 0;
-        cudaDeviceGetLimit(&before, cudaLimitMaxL2FetchGranularity);
-        cudaError_t le = cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t)atoi(v));
-        cudaDeviceGetLimit(&after, cudaLimitMaxL2FetchGranularity);
-        fprintf(stderr, "[maze_b200] L2 fetch granularity %zu -> %zu (rc %d)\n", before, after, (int)le);
     }
     *out = ctx;
     return 0;

@@ -19,7 +19,6 @@ struct maze_ctx {
     double h_lut_invalid[256];
     double h_shaping[4];     // index = (D[prev]-D[cur]) & 3 : 0 -> 0, 1 -> +1, 3 -> -1
     int    num_sms;
-    int    step_ept;        // envs per thread of maze_step (tunable: MAZE_STEP_EPT)
     void*  d_scratch;       // library-owned scratch (candidate wall planes of scored generation), grown on demand
     size_t scratch_bytes;
     void*  net_profile;     // maze_net.cu: in-situ launch timing (events), created on first use

@@ -15,7 +15,6 @@
 //                     TMEM epilogue
 // Everything else (fc3 head, loss, conv weight gradient, transposes, AdamW) is CUDA-core work: < 2 % of the FLOPs.
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include "maze_common.cuh"
 #include "maze_replay.cuh"
@@ -31,28 +30,6 @@ constexpr int GEMM_THREADS = 192;
 enum { EPI_BIAS_ACT = 0, EPI_MASK = 1, EPI_RED_F32 = 2 };
 enum { ACT_NONE = 0, ACT_LRELU = 1, ACT_RELU = 2 };
 constexpr float LRELU_SLOPE = 0.01f;   // nn.LeakyReLU() default (ddqn_agent.py:28,38)
-
-// Every kernel of the train step can be launched with programmatic stream serialization (MAZE_NET_PDL=1): its CTAs may
-// become resident, set up barriers / TMEM / shared memory, and then sit in tc::pdl_wait() until the previous kernel of the
-// stream has finished, so that launch latency and prologue overlap the predecessor's tail.  Measured on the train step it
-// buys nothing (0.489 ms with, 0.483 ms without; the policy forward got slower, 0.093 vs 0.082 ms: early-resident CTAs
-// take shared memory and TMEM from the kernel that is still running), so it is off by default; without the attribute
-// griddepcontrol.wait / launch_dependents are no-ops.
-template <typename... KArgs, typename... Args>
-cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
-    static const bool pdl = [] { const char* e = getenv("MAZE_NET_PDL"); return e && *e && *e != '0'; }();
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = pdl ? 1 : 0;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
-}
 
 struct GemmArgs {
     int M, N, K;          // C[M, N] = A[M, K] . B[N, K]^T
@@ -210,8 +187,6 @@ net_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     tc::tc_fence_before();
     __syncthreads();
     tc::tc_fence_after();
-    tc::pdl_wait();   // nothing above touches global memory
-    tc::pdl_launch();
     const uint32_t tmem_base = tmem_slot;
 
     auto tile_coords = [&](int t, int& m0, int& n0, int& kb_begin, int& nkb) {
@@ -377,8 +352,6 @@ net_gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
     __syncthreads();
     tc::cluster_sync();   // both CTAs' barriers are initialised before anything arrives on them from the peer
     tc::tc_fence_after();
-    tc::pdl_wait();
-    tc::pdl_launch();
     const uint32_t tmem_base = tmem_slot;
 
     if (warp == 0) {
@@ -501,7 +474,8 @@ int launch_gemm_t(maze_ctx* ctx, const bf16* A, int lda, const bf16* B, int ldb,
     ga.splits = splits;
     const int num_tiles = ((g.M + BM - 1) / BM) * ((g.N + BN - 1) / BN) * splits;
     const int grid = num_tiles < ctx->num_sms ? num_tiles : ctx->num_sms;   // persistent: one CTA per SM walks the tiles
-    MAZE_CHECK(launch_pdl(net_gemm_kernel<BN, EPI, MN>, dim3(grid), dim3(GEMM_THREADS), GemmCfg<BN>::SMEM, st, ta, tb, tc_out, ga));
+    net_gemm_kernel<BN, EPI, MN><<<grid, GEMM_THREADS, GemmCfg<BN>::SMEM, st>>>(ta, tb, tc_out, ga);
+    MAZE_CHECK(cudaGetLastError());
     return 0;
 }
 
@@ -515,7 +489,8 @@ int launch_gemm_pair(maze_ctx* ctx, const bf16* A, int lda, const bf16* B, int l
     const int num_tiles = ((g.M + 255) / 256) * ((g.N + 255) / 256);
     int pairs = ctx->num_sms / 2;
     if (num_tiles < pairs) pairs = num_tiles;
-    MAZE_CHECK(launch_pdl(net_gemm_pair_kernel<EPI>, dim3(2 * pairs), dim3(GEMM_THREADS), PAIR_SMEM, st, ta, tb, tc_out, g));
+    net_gemm_pair_kernel<EPI><<<2 * pairs, GEMM_THREADS, PAIR_SMEM, st>>>(ta, tb, tc_out, g);
+    MAZE_CHECK(cudaGetLastError());
     return 0;
 }
 
@@ -578,8 +553,6 @@ __device__ __forceinline__ uint32_t r_offset(int row, int chunk) {   // byte off
 // K-major no-swizzle core-matrix layout; run by maze_dqn_net_refresh.
 __global__ void __launch_bounds__(256)
 net_conv_image_kernel(const float* __restrict__ conv_w, uint8_t* __restrict__ image) {
-    tc::pdl_wait();
-    tc::pdl_launch();
     for (int i = threadIdx.x; i < 3 * 32 * 16; i += 256) {
         const int dy = i / 512, o = (i >> 4) & 31, kk = i & 15;
         float w = 0.f;
@@ -609,8 +582,6 @@ net_features_kernel(const float* __restrict__ vec, const uint32_t* __restrict__ 
         tc::tmem_relinquish();
     }
     for (int i = tid * 16; i < FEAT_R_BYTES; i += FEAT_THREADS * 16) *reinterpret_cast<uint4*>(sR + i) = make_uint4(0, 0, 0, 0);
-    tc::pdl_wait();
-    tc::pdl_launch();
     // weight slices sW[dy][o][kk] = conv_w[o][c][dy][dx], kk = c * 3 + dx, already in the operand layout: net_conv_image_kernel
     // builds the 3 KB image once per weight update (a CTA lives for about seven iterations: building it here from the fp32
     // weights was 12 % of this kernel's time, ncu r02t)
@@ -792,8 +763,6 @@ __device__ __forceinline__ float warp_sum(float v) {
 __global__ void __launch_bounds__(HEAD_THREADS)
 net_head_q_kernel(const bf16* __restrict__ h2, int n, const float* __restrict__ w3, const float* __restrict__ b3, float* __restrict__ q) {
     __shared__ __align__(16) float sw[4 * NET_H2];
-    tc::pdl_wait();
-    tc::pdl_launch();
     for (int i = threadIdx.x; i < 4 * NET_H2; i += HEAD_THREADS) sw[i] = w3[i];
     __syncthreads();
     const int lane = threadIdx.x & 31;
@@ -826,8 +795,6 @@ net_head_loss_kernel(const bf16* __restrict__ h2_s, const bf16* __restrict__ h2_
     __shared__ float sgb[4], sloss;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     float* const sgw = sgw_all + warp * (4 * NET_H2);
-    tc::pdl_wait();
-    tc::pdl_launch();
     // the first sample's rows are requested before the weights: the two round trips to memory overlap
     const int stride = gridDim.x * (HEAD_THREADS / 32);
     int s = blockIdx.x * (HEAD_THREADS / 32) + warp;
@@ -927,8 +894,6 @@ constexpr int COLSUM_COLS = 256, COLSUM_ROWS = 64;
 __global__ void __launch_bounds__(256)
 net_colsum_kernel(const bf16* __restrict__ in, int R, int C, int ld, float* __restrict__ out) {
     __shared__ float part[8][COLSUM_COLS];
-    tc::pdl_wait();
-    tc::pdl_launch();
     const int c0 = blockIdx.x * COLSUM_COLS, r0 = blockIdx.y * COLSUM_ROWS;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int c = c0 + 8 * lane;
@@ -960,61 +925,8 @@ net_colsum_kernel(const bf16* __restrict__ in, int R, int C, int ld, float* __re
 }
 
 // ------------------------------------------------------------------------------------------------------
-// Convolution weight / bias gradient from dL/dX (conv part), the saved pool choices and the packed windows.
-// Thread (o, sub): output channel o, pooled positions sub, sub + 8, ...; 27 tap accumulators in registers.
-__global__ void __launch_bounds__(256)
-net_conv_bwd_kernel(const bf16* __restrict__ dX, const uint8_t* __restrict__ pool_idx, const uint32_t* __restrict__ win, int n,
-                    float* __restrict__ gconv_w, float* __restrict__ gconv_b) {
-    __shared__ uint32_t sw[2][MAZE_WINDOW_WORDS];
-    const int o = threadIdx.x >> 3, sub = threadIdx.x & 7;
-    float acc[27];
-#pragma unroll
-    for (int k = 0; k < 27; ++k) acc[k] = 0.f;
-    float accb = 0.f;
-    int buf = 0;
-    for (int s = blockIdx.x; s < n; s += gridDim.x, buf ^= 1) {
-        if (threadIdx.x < MAZE_WINDOW_WORDS) sw[buf][threadIdx.x] = win[(size_t)s * MAZE_WINDOW_WORDS + threadIdx.x];
-        __syncthreads();   // double-buffered: the previous sample's readers are at most one iteration behind
-        const bf16* grow = dX + (size_t)s * NET_IN + o * 49;
-        const uint8_t* irow = pool_idx + (size_t)s * NET_CONV_OUT + o * 49;
-        for (int q = sub; q < 49; q += 8) {
-            float gq = __bfloat162float(grow[q]);
-            if (gq == 0.f) continue;
-            const uint32_t b = irow[q];
-            if (!(b & 4u)) gq *= LRELU_SLOPE;
-            const int y = 2 * (q / 7) + (int)((b >> 1) & 1u), x = 2 * (q % 7) + (int)(b & 1u);
-            accb += gq;
-#pragma unroll
-            for (int c = 0; c < 3; ++c)
-#pragma unroll
-                for (int dy = 0; dy < 3; ++dy) {
-                    const int iy = y + dy - 1;
-                    uint32_t t3 = 0;
-                    if (iy >= 0 && iy < MAZE_WINDOW) {
-                        const uint32_t rowbits = (sw[buf][c * 8 + (iy >> 1)] >> ((iy & 1) * 16)) & 0x7fffu;
-                        t3 = ((rowbits << 1) >> x) & 7u;
-                    }
-#pragma unroll
-                    for (int dx = 0; dx < 3; ++dx) acc[c * 9 + dy * 3 + dx] += ((t3 >> dx) & 1u) ? gq : 0.f;
-                }
-        }
-    }
-#pragma unroll
-    for (int k = 0; k < 27; ++k) {
-        float v = acc[k];
-        v += __shfl_xor_sync(0xffffffffu, v, 1);
-        v += __shfl_xor_sync(0xffffffffu, v, 2);
-        v += __shfl_xor_sync(0xffffffffu, v, 4);
-        if (sub == 0 && v != 0.f) atomicAdd(gconv_w + o * 27 + k, v);
-    }
-    accb += __shfl_xor_sync(0xffffffffu, accb, 1);
-    accb += __shfl_xor_sync(0xffffffffu, accb, 2);
-    accb += __shfl_xor_sync(0xffffffffu, accb, 4);
-    if (sub == 0 && accb != 0.f) atomicAdd(gconv_b + o, accb);
-}
-
-// ------------------------------------------------------------------------------------------------------
-// The same gradient on the tensor cores.  Per sample
+// Convolution weight / bias gradient from dL/dX (conv part), the saved pool choices and the packed windows, on the
+// tensor cores.  Per sample
 //   D[o, kk] += sum_p A[o, p] * B[kk, p],   p = y * 16 + x over the 16 x 16 padded window positions (K = 256)
 //   A[o, p]  = dL/d(conv output o at p): the pooled gradient dX[o, q] * LeakyReLU', routed to its max-pool winner
 //   B[kk, p] = window bit of tap kk = c * 9 + dy * 3 + dx at p (the window shifted by (dy - 1, dx - 1));
@@ -1061,8 +973,6 @@ net_conv_bwd_tc_kernel(const bf16* __restrict__ dX, const uint8_t* __restrict__ 
     tc::tc_fence_before();
     __syncthreads();
     tc::tc_fence_after();
-    tc::pdl_wait();
-    tc::pdl_launch();
     const uint32_t tmem_base = tmem_slot;
     const uint32_t bar_a = tc::smem_u32(&bar);
     // A units of this thread: channel o, pooled row py, half h (14 units per channel over 8 thread groups)
@@ -1200,8 +1110,6 @@ __global__ void __launch_bounds__(256)
 net_adamw_kernel(float* __restrict__ p, float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, int count, float lr, float beta1,
                  float beta2, float eps, float wd, float bc1, float bc2_sqrt, float grad_scale, float clamp) {
     const int i = (blockIdx.x * 256 + threadIdx.x) * 4;
-    tc::pdl_wait();
-    tc::pdl_launch();
     if (i >= count) return;
     float4 P = *reinterpret_cast<float4*>(p + i), G = *reinterpret_cast<float4*>(g + i), M = *reinterpret_cast<float4*>(m + i),
            V = *reinterpret_cast<float4*>(v + i);
@@ -1230,8 +1138,6 @@ net_adamw_kernel(float* __restrict__ p, float* __restrict__ g, float* __restrict
 __global__ void __launch_bounds__(256)
 net_refresh_kernel(const float* __restrict__ w, int R, int C, bf16* __restrict__ wb, bf16* __restrict__ wt) {
     __shared__ float tile[32][33];
-    tc::pdl_wait();
-    tc::pdl_launch();
     const int r0 = blockIdx.y * 32, c0 = blockIdx.x * 32;
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
     for (int i = ty; i < 32; i += 8) {
@@ -1342,17 +1248,6 @@ int auto_splits(int base_tiles, int nkb, int sms) {
     return best;
 }
 
-// Rows per forward chunk of maze_dqn_backward (MAZE_NET_CHUNK_ROWS; a multiple of 256; 0 = the whole batch at once).
-int fc_chunk_rows() {
-    static const int rows = [] {
-        const char* e = getenv("MAZE_NET_CHUNK_ROWS");
-        int v = e && *e ? atoi(e) : 0;
-        if (v <= 0) v = 1 << 30;
-        return (v + 255) / 256 * 256;
-    }();
-    return rows;
-}
-
 // In-situ kernel times: while enabled (maze_dqn_net_profile), maze_dqn_backward records a CUDA event on its stream after
 // every launch; maze_dqn_net_profile_read turns the last call's events into per-launch durations.  These are the times
 // the kernels take INSIDE the train step (warm L2, real clocks), which ncu's serialised cold-cache replays do not show.
@@ -1385,18 +1280,15 @@ int features(maze_ctx* ctx, bool save_idx, const float* vec, const uint32_t* win
              uint8_t* idx, cudaStream_t st) {
     const int pairs = (n + 1) / 2;   // two samples per iteration
     const int grid = pairs < ctx->num_sms * 4 ? pairs : ctx->num_sms * 4;   // 128 TMEM columns per CTA: four CTAs per SM
-    MAZE_CHECK(launch_pdl(save_idx ? net_features_kernel<true> : net_features_kernel<false>, dim3(grid), dim3(FEAT_THREADS), 0, st, vec, win, n,
-                          reinterpret_cast<const uint4*>(conv_image), params + MAZE_NET_OFF_CONV_B, X, idx));
+    const auto kernel = save_idx ? net_features_kernel<true> : net_features_kernel<false>;
+    kernel<<<grid, FEAT_THREADS, 0, st>>>(vec, win, n, reinterpret_cast<const uint4*>(conv_image), params + MAZE_NET_OFF_CONV_B, X, idx);
+    MAZE_CHECK(cudaGetLastError());
     prof_mark(ctx, st, save_idx ? "features (conv + pool, saves argmax)" : "features (conv + pool)");
     return 0;
 }
 
-// Tile choice of the four K-major GEMMs of the net: CTA pairs (256 x 256) once there are at least two row blocks;
-// MAZE_NET_NO_PAIRS=1 keeps the single-CTA kernel (A/B measurements).
-int fc_tile(int rows) {
-    static const bool no_pairs = [] { const char* e = getenv("MAZE_NET_NO_PAIRS"); return e && *e && *e != '0'; }();
-    return rows > 128 && !no_pairs ? 512 : 256;
-}
+// Tile choice of the four K-major GEMMs of the net: CTA pairs (256 x 256) once there are at least two row blocks.
+int fc_tile(int rows) { return rows > 128 ? 512 : 256; }
 
 // X [rows, 1600] -> h1 [rows, 1024] -> h2 [rows, 512] with one net's weights
 int mlp_forward(maze_ctx* ctx, const bf16* X, int rows, const bf16* w1b, const bf16* w2b, const float* params, bf16* h1, bf16* h2, cudaStream_t st) {
@@ -1444,9 +1336,9 @@ extern "C" int maze_dqn_net_refresh(maze_ctx* ctx, const maze_dqn_net* net, int 
     bf16* w2b = reinterpret_cast<bf16*>(which ? net->tw2_bf16 : net->w2_bf16);
     bf16* w1t = which ? nullptr : reinterpret_cast<bf16*>(net->w1t_bf16);
     bf16* w2t = which ? nullptr : reinterpret_cast<bf16*>(net->w2t_bf16);
-    MAZE_CHECK(launch_pdl(net_refresh_kernel, dim3(NET_IN / 32, NET_H1 / 32), dim3(256), 0, st, p + MAZE_NET_OFF_W1, NET_H1, NET_IN, w1b, w1t));
-    MAZE_CHECK(launch_pdl(net_refresh_kernel, dim3(NET_H1 / 32, NET_H2 / 32), dim3(256), 0, st, p + MAZE_NET_OFF_W2, NET_H2, NET_H1, w2b, w2t));
-    MAZE_CHECK(launch_pdl(net_conv_image_kernel, dim3(1), dim3(256), 0, st, p + MAZE_NET_OFF_CONV_W, carve(net->workspace, net->max_batch).conv_image[which]));
+    net_refresh_kernel<<<dim3(NET_IN / 32, NET_H1 / 32), 256, 0, st>>>(p + MAZE_NET_OFF_W1, NET_H1, NET_IN, w1b, w1t);
+    net_refresh_kernel<<<dim3(NET_H1 / 32, NET_H2 / 32), 256, 0, st>>>(p + MAZE_NET_OFF_W2, NET_H2, NET_H1, w2b, w2t);
+    net_conv_image_kernel<<<1, 256, 0, st>>>(p + MAZE_NET_OFF_CONV_W, carve(net->workspace, net->max_batch).conv_image[which]);
     MAZE_CHECK(cudaGetLastError());
     return 0;
 }
@@ -1477,7 +1369,8 @@ extern "C" int maze_dqn_forward(maze_ctx* ctx, const maze_dqn_net* net, int whic
                              reinterpret_cast<const bf16*>(which ? net->tw2_bf16 : net->w2_bf16), p, w.h1, w.h2, st))
         return rc;
     const int grid = (n + 7) / 8 < ctx->num_sms * 4 ? (n + 7) / 8 : ctx->num_sms * 4;
-    MAZE_CHECK(launch_pdl(net_head_q_kernel, dim3(grid), dim3(HEAD_THREADS), 0, st, w.h2, n, p + MAZE_NET_OFF_W3, p + MAZE_NET_OFF_B3, q_out));
+    net_head_q_kernel<<<grid, HEAD_THREADS, 0, st>>>(w.h2, n, p + MAZE_NET_OFF_W3, p + MAZE_NET_OFF_B3, q_out);
+    MAZE_CHECK(cudaGetLastError());
     return 0;
 }
 
@@ -1497,38 +1390,29 @@ extern "C" int maze_dqn_backward(maze_ctx* ctx, const maze_dqn_net* net, const f
     const bf16 *w1t = reinterpret_cast<const bf16*>(net->w1t_bf16), *w2t = reinterpret_cast<const bf16*>(net->w2t_bf16);
     prof_reset(ctx, st);
     MAZE_CHECK(cudaMemsetAsync(net->loss, 0, sizeof(float), st));
-    // forward: source net on states and next states, target net on next states.  Done in row chunks -- features, fc1, fc2 of
-    // one chunk back to back -- so that a chunk's X (3.2 KB a row) and h1 (2 KB a row) are still in L2 when the next GEMM
-    // reads them: with whole-batch passes (n = 8192: 52 MB of X, 33 MB of h1) the GEMMs ran at their cold-cache time in
-    // situ, twice the L2-warm one (tools/net_selftest.py profile; DESIGN.md 4.3).
+    // forward: source net on states and next states, target net on next states
     bf16* Xt = w.dX;   // the target net has its own conv weights, so its own features; dX is free until the backward-data GEMM
     const bf16 *tw1b = reinterpret_cast<const bf16*>(net->tw1_bf16), *tw2b = reinterpret_cast<const bf16*>(net->tw2_bf16);
-    const int chunk = fc_chunk_rows();
-    for (int r0 = 0; r0 < n; r0 += chunk) {
-        const int rows = n - r0 < chunk ? n - r0 : chunk;
-        const float *v0 = vec + (size_t)r0 * 6, *v1 = next_vec + (size_t)r0 * 6;
-        const uint32_t *w0 = win + (size_t)r0 * MAZE_WINDOW_WORDS, *w1 = next_win + (size_t)r0 * MAZE_WINDOW_WORDS;
-        const size_t a = (size_t)r0, b = np + (size_t)r0;
-        if (int rc = features(ctx, true, v0, w0, rows, p, w.conv_image[0], w.X + a * NET_IN, w.idx + a * NET_CONV_OUT, st)) return rc;
-        if (int rc = mlp_forward(ctx, w.X + a * NET_IN, rows, w1b, w2b, p, w.h1 + a * NET_H1, w.h2 + a * NET_H2, st)) return rc;
-        if (int rc = features(ctx, false, v1, w1, rows, p, w.conv_image[0], w.X + b * NET_IN, nullptr, st)) return rc;
-        if (int rc = mlp_forward(ctx, w.X + b * NET_IN, rows, w1b, w2b, p, w.h1 + b * NET_H1, w.h2 + b * NET_H2, st)) return rc;
-        if (int rc = features(ctx, false, v1, w1, rows, net->target, w.conv_image[1], Xt + a * NET_IN, nullptr, st)) return rc;
-        if (int rc = mlp_forward(ctx, Xt + a * NET_IN, rows, tw1b, tw2b, net->target, w.h1t_tn + a * NET_H1, w.h2_tn + a * NET_H2, st)) return rc;
-    }
+    if (int rc = features(ctx, true, vec, win, n, p, w.conv_image[0], w.X, w.idx, st)) return rc;
+    if (int rc = mlp_forward(ctx, w.X, n, w1b, w2b, p, w.h1, w.h2, st)) return rc;
+    if (int rc = features(ctx, false, next_vec, next_win, n, p, w.conv_image[0], w.X + np * NET_IN, nullptr, st)) return rc;
+    if (int rc = mlp_forward(ctx, w.X + np * NET_IN, n, w1b, w2b, p, w.h1 + np * NET_H1, w.h2 + np * NET_H2, st)) return rc;
+    if (int rc = features(ctx, false, next_vec, next_win, n, net->target, w.conv_image[1], Xt, nullptr, st)) return rc;
+    if (int rc = mlp_forward(ctx, Xt, n, tw1b, tw2b, net->target, w.h1t_tn, w.h2_tn, st)) return rc;
     {
         const int grid = (n + 7) / 8 < 2 * ctx->num_sms ? (n + 7) / 8 : 2 * ctx->num_sms;   // two CTAs per SM; the fc3 gradient is merged with one atomic per CTA and entry
         MAZE_CHECK(cudaFuncSetAttribute(net_head_loss_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)HEAD_LOSS_SMEM));
-        MAZE_CHECK(launch_pdl(net_head_loss_kernel, dim3(grid), dim3(HEAD_THREADS), HEAD_LOSS_SMEM, st, w.h2, w.h2 + np * NET_H2, w.h2_tn, n, p + MAZE_NET_OFF_W3,
-                              p + MAZE_NET_OFF_B3, net->target + MAZE_NET_OFF_W3, net->target + MAZE_NET_OFF_B3, action, reward, gamma, w.dh2,
-                              gr + MAZE_NET_OFF_W3, gr + MAZE_NET_OFF_B3, net->loss, qsa_out));
+        net_head_loss_kernel<<<grid, HEAD_THREADS, HEAD_LOSS_SMEM, st>>>(w.h2, w.h2 + np * NET_H2, w.h2_tn, n, p + MAZE_NET_OFF_W3, p + MAZE_NET_OFF_B3,
+                                                                         net->target + MAZE_NET_OFF_W3, net->target + MAZE_NET_OFF_B3, action, reward, gamma,
+                                                                         w.dh2, gr + MAZE_NET_OFF_W3, gr + MAZE_NET_OFF_B3, net->loss, qsa_out);
+        MAZE_CHECK(cudaGetLastError());
         prof_mark(ctx, st, "head: Q, double-Q target, loss, dQ, fc3 gradients");
     }
     // fc2: dW2 = dh2^T . h1 (MN-major operands: straight from the [n, features] activations), db2 = colsum(dh2),
     //      dh1 = (dh2 . W2) * LeakyReLU'(h1)
     const int nkb_n = (n + BK - 1) / BK;
-    MAZE_CHECK(launch_pdl(net_colsum_kernel, dim3(NET_H2 / COLSUM_COLS, (n + COLSUM_ROWS - 1) / COLSUM_ROWS), dim3(256), 0, st, w.dh2, n, NET_H2, NET_H2,
-                          gr + MAZE_NET_OFF_B2));
+    net_colsum_kernel<<<dim3(NET_H2 / COLSUM_COLS, (n + COLSUM_ROWS - 1) / COLSUM_ROWS), 256, 0, st>>>(w.dh2, n, NET_H2, NET_H2, gr + MAZE_NET_OFF_B2);
+    MAZE_CHECK(cudaGetLastError());
     prof_mark(ctx, st, "fc2 bias gradient (column sums)");
     GemmArgs g{};
     g.M = NET_H2; g.N = NET_H1; g.K = n; g.C = gr + MAZE_NET_OFF_W2; g.ldc = NET_H1;
@@ -1539,8 +1423,8 @@ extern "C" int maze_dqn_backward(maze_ctx* ctx, const maze_dqn_net* net, const f
     if (int rc = launch_gemm(ctx, EPI_MASK, fc_tile(n), w.dh2, NET_H2, w2t, NET_H2, g, 1, st)) return rc;
     prof_mark(ctx, st, "fc2 backward-data GEMM (masked)");
     // fc1: dW1 = dh1^T . X, db1 = colsum(dh1), dX = dh1 . W1
-    MAZE_CHECK(launch_pdl(net_colsum_kernel, dim3(NET_H1 / COLSUM_COLS, (n + COLSUM_ROWS - 1) / COLSUM_ROWS), dim3(256), 0, st, w.dh1, n, NET_H1, NET_H1,
-                          gr + MAZE_NET_OFF_B1));
+    net_colsum_kernel<<<dim3(NET_H1 / COLSUM_COLS, (n + COLSUM_ROWS - 1) / COLSUM_ROWS), 256, 0, st>>>(w.dh1, n, NET_H1, NET_H1, gr + MAZE_NET_OFF_B1);
+    MAZE_CHECK(cudaGetLastError());
     prof_mark(ctx, st, "fc1 bias gradient (column sums)");
     g = GemmArgs{};
     g.M = NET_H1; g.N = NET_IN; g.K = n; g.C = gr + MAZE_NET_OFF_W1; g.ldc = NET_IN;
@@ -1553,16 +1437,11 @@ extern "C" int maze_dqn_backward(maze_ctx* ctx, const maze_dqn_net* net, const f
     g.M = n; g.N = NET_CONV_OUT; g.K = NET_H1; g.C = w.dX; g.ldc = NET_IN; g.act = ACT_NONE;
     if (int rc = launch_gemm(ctx, EPI_BIAS_ACT, fc_tile(n), w.dh1, NET_H1, w1t, NET_H1, g, 1, st)) return rc;
     prof_mark(ctx, st, "fc1 backward-data GEMM");
-    static const bool conv_bwd_cuda_cores = getenv("MAZE_NET_CONV_BWD_CUDA_CORES") != nullptr;   // A/B switch for the CUDA-core version
-    if (conv_bwd_cuda_cores) {
-        const int grid = n < ctx->num_sms * 4 ? n : ctx->num_sms * 4;
-        net_conv_bwd_kernel<<<grid, 256, 0, st>>>(w.dX, w.idx, win, n, gr + MAZE_NET_OFF_CONV_W, gr + MAZE_NET_OFF_CONV_B);
-        MAZE_CHECK(cudaGetLastError());
-    } else {
+    {
         MAZE_CHECK(cudaFuncSetAttribute(net_conv_bwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CB_SMEM));
         const int grid = n < ctx->num_sms * 3 ? n : ctx->num_sms * 3;   // 48 KB of operands + 9 KB of staging per CTA: three fit an SM
-        MAZE_CHECK(launch_pdl(net_conv_bwd_tc_kernel, dim3(grid), dim3(CB_THREADS), CB_SMEM, st, w.dX, w.idx, win, n, gr + MAZE_NET_OFF_CONV_W,
-                              gr + MAZE_NET_OFF_CONV_B));
+        net_conv_bwd_tc_kernel<<<grid, CB_THREADS, CB_SMEM, st>>>(w.dX, w.idx, win, n, gr + MAZE_NET_OFF_CONV_W, gr + MAZE_NET_OFF_CONV_B);
+        MAZE_CHECK(cudaGetLastError());
     }
     prof_mark(ctx, st, "conv gradient (un-pool + implicit GEMM)");
     return 0;
@@ -1611,8 +1490,9 @@ extern "C" int maze_dqn_adamw(maze_ctx* ctx, const maze_dqn_net* net, float lr, 
     if (step < 1) return maze_fail_arg(ctx, MAZE_E_RANGE, "maze_dqn_adamw: step counts from 1");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const float bc1 = 1.f - powf(beta1, (float)step), bc2 = 1.f - powf(beta2, (float)step);
-    MAZE_CHECK(launch_pdl(net_adamw_kernel, dim3((MAZE_NET_PARAMS / 4 + 255) / 256), dim3(256), 0, st, net->params, net->grads, net->adam_m, net->adam_v,
-                          (int)MAZE_NET_PARAMS, lr, beta1, beta2, eps, weight_decay, bc1, sqrtf(bc2), grad_scale, clamp));
+    net_adamw_kernel<<<(MAZE_NET_PARAMS / 4 + 255) / 256, 256, 0, st>>>(net->params, net->grads, net->adam_m, net->adam_v, (int)MAZE_NET_PARAMS, lr, beta1,
+                                                                       beta2, eps, weight_decay, bc1, sqrtf(bc2), grad_scale, clamp);
+    MAZE_CHECK(cudaGetLastError());
     return maze_dqn_net_refresh(ctx, net, 0, stream);
 }
 

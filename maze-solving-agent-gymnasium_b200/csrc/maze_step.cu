@@ -1,6 +1,6 @@
 // Env step / reset kernels (sm_100a).
 //
-// One thread per env (optionally 2-4 envs per thread).  State is one packed 64-bit word per env
+// One env per thread (two per thread from 64 K envs up).  State is one packed 64-bit word per env
 // (coalesced 8-byte load/store); the maze is read through its one-byte-per-block step table
 // (L2/L1 resident for a maze pool); the only scattered DRAM access is the 2-byte visit counter of
 // the block stepped onto, fetched only for legal moves, from a cell-major array.
@@ -13,9 +13,6 @@ constexpr int STEP_THREADS = 256;
 #ifndef MAZE_STEP_MINB1
 #define MAZE_STEP_MINB1 6
 #endif
-#ifndef MAZE_STEP_MINB4
-#define MAZE_STEP_MINB4 2
-#endif
 #ifndef MAZE_STEP_MINB2
 #define MAZE_STEP_MINB2 5
 #endif
@@ -26,7 +23,7 @@ constexpr int STEP_THREADS = 256;
 // counter is only fetched when the move is legal (a wall hit needs no counter), which matters
 // because every such fetch costs a whole DRAM line.
 template <int EPT, bool kStats, bool kTiled>
-__global__ void __launch_bounds__(STEP_THREADS, EPT == 2 ? MAZE_STEP_MINB2 : (EPT == 1 ? MAZE_STEP_MINB1 : MAZE_STEP_MINB4))
+__global__ void __launch_bounds__(STEP_THREADS, EPT == 2 ? MAZE_STEP_MINB2 : MAZE_STEP_MINB1)
 maze_step_kernel(maze_env_batch b, const uint8_t* __restrict__ actions, uint32_t mode, StepLuts luts) {
     const int base = blockIdx.x * (STEP_THREADS * EPT) + threadIdx.x;
 
@@ -370,8 +367,7 @@ extern "C" int maze_step(maze_ctx* ctx, const maze_env_batch* b, const uint8_t* 
     const StepLuts luts = step_luts(ctx);
     const bool stats = b->ep_return || b->stats || ((mode & MAZE_STEP_WIN_QUEUE) && b->queue);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    int ept = ctx->step_ept;
-    if (b->num_envs < 64 * 1024) ept = 1;   // small batches: more CTAs beats more loads per thread
+    const int ept = b->num_envs < 64 * 1024 ? 1 : 2;   // small batches: more CTAs beats more loads per thread
     auto grid_for = [&](int e) { return (b->num_envs + STEP_THREADS * e - 1) / (STEP_THREADS * e); };
     auto launch = [&](auto kernel, int e) { kernel<<<grid_for(e), STEP_THREADS, 0, st>>>(*b, actions, mode, luts); };
 #define MAZE_STEP_DISPATCH(EPT_)                                                                          \
@@ -380,8 +376,7 @@ extern "C" int maze_step(maze_ctx* ctx, const maze_env_batch* b, const uint8_t* 
         else       { if (tiled) launch(maze_step_kernel<EPT_, false, true>, EPT_); else launch(maze_step_kernel<EPT_, false, false>, EPT_); } \
     } while (0)
     const bool tiled = b->visit_tiled != 0;
-    if (ept >= 4) MAZE_STEP_DISPATCH(4);
-    else if (ept == 2) MAZE_STEP_DISPATCH(2);
+    if (ept == 2) MAZE_STEP_DISPATCH(2);
     else MAZE_STEP_DISPATCH(1);
 #undef MAZE_STEP_DISPATCH
     MAZE_CHECK(cudaGetLastError());

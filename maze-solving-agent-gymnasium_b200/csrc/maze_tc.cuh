@@ -43,12 +43,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
     }
 }
 
-// Programmatic dependent launch: a kernel launched with the programmatic-stream-serialization attribute may become resident
-// while its predecessor in the stream still runs; pdl_wait() blocks until the predecessor has completed and its writes are
-// visible (everything before it may only touch on-chip state), pdl_launch() lets the successor start becoming resident.
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-
 // generic-proxy shared-memory writes -> visible to the async proxy (TMA / tcgen05.mma operand reads)
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 

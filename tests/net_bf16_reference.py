@@ -7,21 +7,21 @@ a store.  What remains between them and the kernels is the order of the fp32 acc
 dyadic grid those sums are exact in any order and the results agree bit for bit.
 
 Rounding points (line numbers of maze_net.cu):
-  * conv weights -> bf16 (net_conv_image_kernel, :587); the conv bias stays fp32 (:618, :704).
-  * W1, W2 -> bf16 (net_refresh_kernel, :1241, :1247); b1, b2, W3, b3 stay fp32.
-  * state vector -> bf16 when it is written into X (net_features_kernel, :721, `xrow[NET_CONV_OUT + tid]`).
-  * features (net_features_kernel, :684-708): the conv sum over the binary window is exact; the 2 x 2 pool takes the
-    FIRST maximum in the scan order (0,0), (0,1), (1,0), (1,1) (`x > m[ch]`, :693); then fp32 bias, LeakyReLU with
-    slope 0.01f, bf16.  idx byte: bit 0 = x parity of the winner, bit 1 = y parity, bit 2 = pre-activation > 0 (:705).
-  * forward GEMM epilogue (epi_bf16_tile, :119-131): h1 = bf16(lrelu(acc + b1)), h2 = bf16(relu(acc + b2)).
-  * fc3 head (net_head_q_kernel / net_head_loss_kernel, :773-906): fp32 W3, b3 on the bf16 h2; double-Q target from
-    the first maximum of the source net's q(s') (:884-887); gq = 2 d / n; dh2 = bf16(h2 > 0 ? gq W3[a] : 0) (:897-898);
-    the fc3 gradients from the bf16 h2 (:902-903).
+  * conv weights -> bf16 (net_conv_image_kernel, :560); the conv bias stays fp32 (:589, :675).
+  * W1, W2 -> bf16 (net_refresh_kernel, :1147, :1153); b1, b2, W3, b3 stay fp32.
+  * state vector -> bf16 when it is written into X (net_features_kernel, :692, `xrow[NET_CONV_OUT + tid]`).
+  * features (net_features_kernel, :655-679): the conv sum over the binary window is exact; the 2 x 2 pool takes the
+    FIRST maximum in the scan order (0,0), (0,1), (1,0), (1,1) (`x > m[ch]`, :664); then fp32 bias, LeakyReLU with
+    slope 0.01f, bf16.  idx byte: bit 0 = x parity of the winner, bit 1 = y parity, bit 2 = pre-activation > 0 (:676).
+  * forward GEMM epilogue (epi_bf16_tile, :96-108): h1 = bf16(lrelu(acc + b1)), h2 = bf16(relu(acc + b2)).
+  * fc3 head (net_head_q_kernel / net_head_loss_kernel, :744-873): fp32 W3, b3 on the bf16 h2; double-Q target from
+    the first maximum of the source net's q(s') (:851-854); gq = 2 d / n; dh2 = bf16(h2 > 0 ? gq W3[a] : 0) (:864-865);
+    the fc3 gradients from the bf16 h2 (:869-870).
   * backward: gb2 = colsum(dh2), dW2 = dh2^T h1; dh1 = bf16((dh2 W2) * (h1 > 0 ? 1 : 0.01f)) with the sign of the
-    STORED bf16 activation, an exact zero taking the slope (EPI_MASK, :133-144); gb1 = colsum(dh1), dW1 = dh1^T X;
-    dX = bf16(dh1 W1) over the 1568 conv columns (EPI_BIAS_ACT without bias, :1552-1554).
-  * conv gradient: dX routed to the pool winner, times LeakyReLU' from idx bit 2.  net_conv_bwd_tc_kernel rounds
-    gv * 0.01f to bf16 before the MMA (:1131-1133, tc=True); net_conv_bwd_kernel keeps it in fp32 (:981-984, tc=False).
+    STORED bf16 activation, an exact zero taking the slope (EPI_MASK, :110-121); gb1 = colsum(dh1), dW1 = dh1^T X;
+    dX = bf16(dh1 W1) over the 1568 conv columns (EPI_BIAS_ACT without bias, :1436-1438).
+  * conv gradient (net_conv_bwd_tc_kernel): dX routed to the pool winner, times LeakyReLU' from idx bit 2; gv * 0.01f
+    is rounded to bf16 before the MMA (:1041-1043).
 
 With rounding=False every rounding point is the identity and the slope is 0.01: the functions then compute the fp32
 net's exact float64 semantics, which tests/test_net_bf16_reference_cpu.py checks against autograd.
@@ -145,13 +145,13 @@ def first_argmax(q):
     return best, (gap > 0) & (gap <= ARGMAX_NEAR_REL * top[:, 0].abs().clamp_min(1e-30))
 
 
-def conv_grad(w: NetWeights, dX, idx, win, tc: bool = True):
+def conv_grad(w: NetWeights, dX, idx, win):
     """d loss / d conv weight [32, 3, 3, 3] and bias [32] from dX [n, 1568], the pool choices and the windows."""
     r, n = w.r, dX.shape[0]
     g = dX.view(n, 32, 49)
     b = idx.view(n, 32, 49)
     neg = r.f32(g * r.slope)
-    gv = torch.where((b & 4) != 0, g, r.bf16(neg) if tc else neg)
+    gv = torch.where((b & 4) != 0, g, r.bf16(neg))
     q = torch.arange(49, device=dX.device)
     y = 2 * (q // 7) + ((b >> 1) & 1).long()
     x = 2 * (q % 7) + (b & 1).long()
@@ -161,8 +161,7 @@ def conv_grad(w: NetWeights, dX, idx, win, tc: bool = True):
     return gw, G.sum((0, 2))
 
 
-def ddqn_backward(src: NetWeights, tgt: NetWeights, vec, win, next_vec, next_win, action, reward, gamma: float, tc: bool = True,
-                  keep=None):
+def ddqn_backward(src: NetWeights, tgt: NetWeights, vec, win, next_vec, next_win, action, reward, gamma: float, keep=None):
     """maze_dqn_backward: loss, q(s, a) and the gradients of the source net (state_dict names and shapes).
     keep: optional [n] 0/1 weights on the samples' gradient contributions (1 / n stays the batch's), to model a kernel
     that lost some samples."""
@@ -189,7 +188,7 @@ def ddqn_backward(src: NetWeights, tgt: NetWeights, vec, win, next_vec, next_win
     gb1 = dh1.sum(0)
     gw1 = dh1.t() @ X
     dX = r.bf16(dh1 @ src.w1[:, :1568])
-    gcw, gcb = conv_grad(src, dX, fs["idx"], win, tc=tc)
+    gcw, gcb = conv_grad(src, dX, fs["idx"], win)
     grads = {"conv.0.weight": gcw, "conv.0.bias": gcb, "fc.0.weight": gw1, "fc.0.bias": gb1, "fc.2.weight": gw2, "fc.2.bias": gb2,
              "fc.4.weight": gw3, "fc.4.bias": gb3}
     return dict(loss=loss, qsa=qsa, grads=grads, dh2=dh2, dh1=dh1, dX=dX, best=best, argmax_near=argmax_near, fs=fs, fn=fn, ft=ft)

@@ -2,7 +2,7 @@
 bit for bit where the operands make every fp32 sum exact, and at the production batch (n = 8192) with tolerances an
 order of magnitude tighter than test_gpu_net.py's, tight enough to see one lost 128-sample tile.
 
-Measured on a B200 (1000 W power limit), worst case over every parameter set and switch; TOL holds the bounds:
+Measured on a B200 (1000 W power limit), worst case over every parameter set; TOL holds the bounds:
   forward q: row error / max |q|                       2.0e-3   (TOL 5e-3)
   q(s, a): error / max |q(s, a)|                       1.6e-3   (TOL 4e-3)
   loss: relative                                       9.5e-5   (TOL 3e-4)
@@ -11,10 +11,6 @@ Measured on a B200 (1000 W power limit), worst case over every parameter set and
   AdamW parameters: error / lr                         2.9e-5   (TOL 1e-4)
   features with the default init: bit-exact (no entry 1 ulp off, no pool choice different)
 """
-import os
-import subprocess
-import sys
-
 import numpy as np
 import pytest
 
@@ -24,7 +20,6 @@ pytestmark = pytest.mark.gpu
 import net_bf16_reference as nbr  # noqa: E402
 from net_reference import pack_windows  # noqa: E402
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SMS = torch.cuda.get_device_properties(0).multi_processor_count if torch.cuda.is_available() else 148
 
 # Bounds from measurement (see the module docstring).  A gradient passes at relative Frobenius error <= TOL[name] and no
@@ -97,9 +92,9 @@ def _check_grad(name, got, ref, what):
     assert rel <= TOL[name] and worst <= WORST_FACTOR * TOL[name], f"{what} {name}: relative Frobenius error {rel:.3g}, worst entry {worst:.3g} (tol {TOL[name]})"
 
 
-def _reference_backward(sd_src, sd_tgt, b, gamma=0.9, tc=True, keep=None):
+def _reference_backward(sd_src, sd_tgt, b, gamma=0.9, keep=None):
     return nbr.ddqn_backward(_weights(sd_src), _weights(sd_tgt), b["vec"], b["win"], b["nvec"], b["nwin"], b["action"], b["reward"], gamma,
-                             tc=tc, keep=keep)
+                             keep=keep)
 
 
 def _check_backward(loss, qsa, grads_flat, ref, what):
@@ -128,7 +123,7 @@ def _check_backward(loss, qsa, grads_flat, ref, what):
 # Operands are k / 8 (|k| <= 8), bias and accumulated-onto C multiples of 1 / 64 in [-1, 1]: every product is a multiple
 # of 1 / 64 and every partial sum s satisfies |s| * 64 <= (K + 2) * 64 < 2^24 (K <= 8200), so fp32 holds every partial sum
 # exactly, in any order and over any split-K partition, and C must equal the float64 result rounded as the epilogue
-# rounds (maze_net.cu:119-143).
+# rounds (maze_net.cu:96-120).
 def _grid(shape, g, denom=8, lim=8):
     return (torch.randint(-lim, lim + 1, shape, generator=g).double() / denom).cuda()
 
@@ -349,92 +344,7 @@ def test_double_q_exact_tie_takes_the_first_action():
     assert abs(other - ref["loss"].item()) > 10 * TOL["loss"] * ref["loss"].item()
 
 
-# ---- e. the A/B switches, each in a process of its own (the kernels read them once per process) ---------------------
-def _child_main(out, ns, adam_step):
-    """Run in a subprocess: backward (and forward) at each n on a fixed net and batches; with adam_step also AdamW, then
-    a second backward with the updated weights.  Writes the results to `out` (.npz)."""
-    net = _make_net(max(ns))
-    res = {}
-    for n in ns:
-        b = _batch(n, 4000 + n)
-        loss, qsa, grads = _run_backward(net, b)
-        res[f"loss{n}"], res[f"qsa{n}"], res[f"grads{n}"] = np.float64(loss), qsa.cpu().numpy(), grads.cpu().numpy()
-        res[f"q{n}"] = net.forward(b["vec"], b["pwin"]).cpu().numpy()
-    if adam_step:
-        n = ns[-1]
-        net.backward(b["vec"], b["pwin"], b["nvec"], b["pnwin"], b["action"], b["reward"], 0.9)   # grads accumulate: 2 x
-        res["grads_acc"] = net.grads.cpu().numpy()
-        net.adamw(1e-3, grad_scale=0.5)
-        res["params1"], res["m1"], res["v1"] = net.params.cpu().numpy(), net.adam_m.cpu().numpy(), net.adam_v.cpu().numpy()
-        b2 = _batch(n, 9000)
-        loss, qsa, grads = _run_backward(net, b2)
-        res["loss_2"], res["qsa_2"], res["grads_2"] = np.float64(loss), qsa.cpu().numpy(), grads.cpu().numpy()
-    torch.cuda.synchronize()
-    np.savez(out, **res)
-
-
-def _run_child(tmp_path, env, ns, adam_step=False):
-    out = str(tmp_path / "out.npz")
-    code = (f"import test_gpu_net_exact as t; t._child_main({out!r}, {list(ns)!r}, {adam_step!r})")
-    e = dict(os.environ)
-    e.update(env)
-    e["PYTHONPATH"] = os.pathsep.join([os.path.join(ROOT, "tests"), ROOT, os.path.join(ROOT, "maze-solving-agent-gymnasium_b200")])
-    p = subprocess.run([sys.executable, "-c", code], env=e, cwd=ROOT, capture_output=True, text=True, timeout=600)
-    assert p.returncode == 0, p.stderr[-3000:]
-    return dict(np.load(out))
-
-
-def _check_child(res, ns, tc=True, what=""):
-    net = _make_net(8)
-    src, tgt = net.state_dict("source"), net.state_dict("target")
-    for n in ns:
-        b = _batch(n, 4000 + n)
-        ref = _reference_backward(src, tgt, b, tc=tc)
-        _check_backward(float(res[f"loss{n}"]), torch.from_numpy(res[f"qsa{n}"]).cuda(), torch.from_numpy(res[f"grads{n}"]).cuda(), ref,
-                        f"{what} n={n}")
-        q = torch.from_numpy(res[f"q{n}"]).cuda().double()
-        assert ((q - ref["fs"]["q"]).abs().max() / ref["fs"]["q"].abs().max()).item() <= TOL["q"]
-    return src, tgt
-
-
-def test_conv_gradient_on_cuda_cores(tmp_path):
-    """MAZE_NET_CONV_BWD_CUDA_CORES=1: net_conv_bwd_kernel, which keeps gv * 0.01f in fp32 (the reference's tc=False)."""
-    ns = [200, 8192]
-    _check_child(_run_child(tmp_path, {"MAZE_NET_CONV_BWD_CUDA_CORES": "1"}, ns), ns, tc=False, what="cuda-core conv gradient")
-
-
-def test_without_cta_pairs(tmp_path):
-    ns = [1000, 8192]
-    _check_child(_run_child(tmp_path, {"MAZE_NET_NO_PAIRS": "1"}, ns), ns, what="no pairs")
-
-
-def test_forward_in_256_row_chunks(tmp_path):
-    """MAZE_NET_CHUNK_ROWS=256: at n = 1000 the last chunk has 232 rows."""
-    ns = [1000, 8192]
-    _check_child(_run_child(tmp_path, {"MAZE_NET_CHUNK_ROWS": "256"}, ns), ns, what="chunks of 256")
-
-
-def test_programmatic_dependent_launch(tmp_path):
-    """MAZE_NET_PDL=1: every kernel of the train step may start before its predecessor has finished and waits in
-    griddepcontrol.wait; one that touched global memory before its wait would race.  Backward, AdamW and a second
-    backward with the refreshed weights, at n = 8192."""
-    n = 8192
-    res = _run_child(tmp_path, {"MAZE_NET_PDL": "1"}, [n], adam_step=True)
-    src, tgt = _check_child(res, [n], what="PDL")
-    # the second backward accumulated onto the first: twice the gradient
-    g1, gacc = torch.from_numpy(res[f"grads{n}"]).cuda(), torch.from_numpy(res["grads_acc"]).cuda()
-    rel, _ = _rel(gacc, 2 * g1)
-    assert rel <= 1e-5, rel
-    p0 = _make_net(8).params
-    p1, m1, v1 = _adamw_reference(p0.double(), gacc.double(), torch.zeros_like(gacc, dtype=torch.float64), torch.zeros_like(gacc, dtype=torch.float64),
-                                  step=1, lr=1e-3, wd=1e-2, grad_scale=0.5, clamp=1.0)
-    _check_adamw(torch.from_numpy(res["params1"]).cuda(), p1, 1e-3, "PDL adamw")
-    b2 = _batch(n, 9000)
-    ref = _reference_backward(_sd_from_flat(torch.from_numpy(res["params1"]).cuda()), tgt, b2)
-    _check_backward(float(res["loss_2"]), torch.from_numpy(res["qsa_2"]).cuda(), torch.from_numpy(res["grads_2"]).cuda(), ref, "PDL step 2")
-
-
-# ---- f. AdamW ----------------------------------------------------------------------------------------------------
+# ---- e. AdamW ----------------------------------------------------------------------------------------------------
 def _f32(x):
     return float(np.float32(x))
 
@@ -479,6 +389,28 @@ def test_adamw_grad_scale_no_clamp_late_step():
     assert ((net.adam_v.double() - v1).abs() <= 1e-6 * (b2 * v0 + (1 - b2) * gr * gr)).all()
     _check_adamw(net.params, p1, 1e-3, "adamw step 10000")
     assert (net.grads == 0).all()
+
+
+def test_accumulated_gradient_adamw_and_next_backward():
+    """At the production batch: a second backward adds its gradient onto the first, AdamW steps from the sum, and the
+    next backward runs on the refreshed weights (the fp32 master copy and the bf16 GEMM operands)."""
+    n = 8192
+    net = _make_net(n)
+    p0 = net.params.double()
+    b = _batch(n, 4000 + n)
+    _, _, g1 = _run_backward(net, b)
+    net.backward(b["vec"], b["pwin"], b["nvec"], b["pnwin"], b["action"], b["reward"], 0.9)
+    gacc = net.grads.double()
+    rel, _ = _rel(gacc, 2 * g1)
+    assert rel <= 1e-5, rel
+    net.adamw(1e-3, grad_scale=0.5)
+    zeros = torch.zeros_like(gacc)
+    p1, _, _ = _adamw_reference(p0, gacc, zeros, zeros, step=1, lr=1e-3, wd=1e-2, grad_scale=0.5, clamp=1.0)
+    _check_adamw(net.params, p1, 1e-3, "adamw from the accumulated gradient")
+    b2 = _batch(n, 9000)
+    loss, qsa, grads = _run_backward(net, b2)
+    ref = _reference_backward(_sd_from_flat(net.params), net.state_dict("target"), b2)
+    _check_backward(loss, qsa, grads, ref, "backward after adamw")
 
 
 def test_padding_columns_stay_zero_over_train_steps():

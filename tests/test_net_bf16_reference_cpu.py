@@ -40,7 +40,7 @@ def test_unrounded_reference_equals_float64_autograd(n):
         err = (got - p.grad).abs().max().item()
         assert err <= 1e-10 * max(1.0, p.grad.abs().max().item()), (name, err)
     # both conv-gradient roundings are the same function without rounding
-    gw, gb = nbr.conv_grad(ws, ref["dX"], ref["fs"]["idx"], win, tc=False)
+    gw, gb = nbr.conv_grad(ws, ref["dX"], ref["fs"]["idx"], win)
     assert torch.equal(gw, ref["grads"]["conv.0.weight"]) and torch.equal(gb, ref["grads"]["conv.0.bias"])
 
 

@@ -281,11 +281,8 @@ def run_case(case):
             by_label[key[1]][1] += 1
         for label, (ms, cnt) in by_label.items():
             lines.append(f"{ms * 1e3:9.1f} us  {cnt:3d} x  {label}")
-        lines.append(f"{total * 1e3:9.1f} us  backward pass, sum of medians over {reps} steps (n = {n}, pairs {'off' if os.environ.get('MAZE_NET_NO_PAIRS') else 'on'}, chunk rows {os.environ.get('MAZE_NET_CHUNK_ROWS', 'default')})")
+        lines.append(f"{total * 1e3:9.1f} us  backward pass, sum of medians over {reps} steps (n = {n})")
         print("\n".join(lines), flush=True)
-        os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-        tag = ("nopairs" if os.environ.get("MAZE_NET_NO_PAIRS") else "pairs") + "_chunk" + os.environ.get("MAZE_NET_CHUNK_ROWS", "default")
-        open(os.path.join(ROOT, "gpurun_out", f"net_insitu_{tag}_n{n}.txt"), "w").write("\n".join(lines) + "\n")
     elif case == "trainloop":   # a short loop for the ncu launch list
         from maze_b200.dqn_net import DQNNet
         n = int(os.environ.get("NET_BATCH", "8192"))
