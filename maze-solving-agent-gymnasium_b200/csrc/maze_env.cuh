@@ -27,71 +27,46 @@ inline StepLuts step_luts(const maze_ctx* ctx) {
 
 // ---- cache-policy helpers --------------------------------------------------------------------
 // What one step touches per env, and how long it is worth keeping in the 126 MB L2:
-//   state word, maze id (12 B)   re-read by the next step          -> MAZE_STATE_POLICY
-//   step table (6.5 KB / maze)   shared by every env of the maze   -> MAZE_TABLE_POLICY
-//   visit counter (2 B RMW)      54 GB array, random access        -> MAZE_VISIT_POLICY
+//   state word, maze id (12 B)   re-read by the next step
+//   step table (6.5 KB / maze)   shared by every env of the maze
+//   visit counter (2 B RMW)      54 GB array, random access
 //   action, obs, reward, flags   written / read once               -> always streaming (.cs)
-// policy values: 0 default, 1 L2 evict_last, 2 L2 evict_first
-#ifndef MAZE_STATE_POLICY
-#define MAZE_STATE_POLICY 1
-#endif
-#ifndef MAZE_TABLE_POLICY
-#define MAZE_TABLE_POLICY 1
-#endif
-#ifndef MAZE_VISIT_POLICY
-#define MAZE_VISIT_POLICY 1
-#endif
-
-template <int kPolicy>
+// The first three are all loaded and stored L2 evict_last.  The default policy and evict_first
+// measured within 2 % of it on B200, except evict_first on the visit sectors, which was 20 %
+// slower: the store misses the sector its own load fetched (DESIGN.md §4.1).
 __device__ __forceinline__ uint64_t l2_policy() {
-    uint64_t p = 0;
-    if (kPolicy == 1) asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-    if (kPolicy == 2) asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
+    uint64_t p;
+    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
     return p;
 }
-template <int kPolicy> __device__ __forceinline__ unsigned long long pol_load(const unsigned long long* p, uint64_t pol) {
-    if (kPolicy == 0) return *p;
+__device__ __forceinline__ unsigned long long pol_load(const unsigned long long* p, uint64_t pol) {
     unsigned long long v;
     asm volatile("ld.global.L2::cache_hint.u64 %0, [%1], %2;" : "=l"(v) : "l"(p), "l"(pol));
     return v;
 }
-template <int kPolicy> __device__ __forceinline__ int pol_load(const int* p, uint64_t pol) {
-    if (kPolicy == 0) return *p;
+__device__ __forceinline__ int pol_load(const int* p, uint64_t pol) {
     int v;
     asm volatile("ld.global.L2::cache_hint.s32 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
     return v;
 }
-template <int kPolicy> __device__ __forceinline__ unsigned pol_load(const uint16_t* p, uint64_t pol) {
-    if (kPolicy == 0) return *p;
+__device__ __forceinline__ unsigned pol_load(const uint16_t* p, uint64_t pol) {
     unsigned short v;
     asm volatile("ld.global.L2::cache_hint.u16 %0, [%1], %2;" : "=h"(v) : "l"(p), "l"(pol));
     return v;
 }
-template <int kPolicy> __device__ __forceinline__ int pol_load_nc(const uint8_t* p, uint64_t pol) {   // read-only data
-    if (kPolicy == 0) return __ldg(p);
+__device__ __forceinline__ int pol_load_nc(const uint8_t* p, uint64_t pol) {   // read-only data
     unsigned v;
     asm volatile("ld.global.nc.L2::cache_hint.u8 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
     return (int)v;
 }
-template <int kPolicy> __device__ __forceinline__ void pol_store(unsigned long long* p, unsigned long long v, uint64_t pol) {
-    if (kPolicy == 0) { *p = v; return; }
+__device__ __forceinline__ void pol_store(unsigned long long* p, unsigned long long v, uint64_t pol) {
     asm volatile("st.global.L2::cache_hint.u64 [%0], %1, %2;" ::"l"(p), "l"(v), "l"(pol) : "memory");
 }
-template <int kPolicy> __device__ __forceinline__ void pol_store(int* p, int v, uint64_t pol) {
-    if (kPolicy == 0) { *p = v; return; }
+__device__ __forceinline__ void pol_store(int* p, int v, uint64_t pol) {
     asm volatile("st.global.L2::cache_hint.s32 [%0], %1, %2;" ::"l"(p), "r"(v), "l"(pol) : "memory");
 }
-template <int kPolicy> __device__ __forceinline__ void pol_store(uint16_t* p, unsigned v, uint64_t pol) {
-    if (kPolicy == 0) { *p = (uint16_t)v; return; }
+__device__ __forceinline__ void pol_store(uint16_t* p, unsigned v, uint64_t pol) {
     asm volatile("st.global.L2::cache_hint.u16 [%0], %1, %2;" ::"l"(p), "h"((unsigned short)v), "l"(pol) : "memory");
-}
-__device__ __forceinline__ unsigned visit_load(const uint16_t* p, uint64_t pol) { return pol_load<MAZE_VISIT_POLICY>(p, pol); }
-#ifndef MAZE_VISIT_STORE_POLICY
-#define MAZE_VISIT_STORE_POLICY MAZE_VISIT_POLICY
-#endif
-__device__ __forceinline__ void visit_store(uint16_t* p, unsigned v, uint64_t pol) {
-    if (MAZE_VISIT_STORE_POLICY == MAZE_VISIT_POLICY) pol_store<MAZE_VISIT_POLICY>(p, v, pol);
-    else pol_store<MAZE_VISIT_STORE_POLICY>(p, v, l2_policy<MAZE_VISIT_STORE_POLICY>());
 }
 
 // index of block (r, c) in an env's visit array (see maze_env_batch.visit_tiled)
@@ -173,9 +148,9 @@ __device__ __forceinline__ StepResult env_transition(const maze_env_batch& b, in
     const int idx = nr * mz.W + nc;
     const int tb = inb ? __ldg(mz.tab + idx) : 0;
     if (inb && (tb & MAZE_TAB_OPEN)) {
-        const uint64_t pol = l2_policy<MAZE_VISIT_POLICY>();
+        const uint64_t pol = l2_policy();
         uint16_t* vp = VISIT_AT(b, e, visit_index(b, nr, nc, mz.W));
-        const unsigned vis = visit_load(vp, pol);
+        const unsigned vis = pol_load(vp, pol);
         const int cnt = ((int)(vis >> 8) == st.epoch) ? (int)(vis & 0xff) : 0;
         if (cnt == 0) {
             if ((nr | (nc << 16)) == mz.goal) {
@@ -188,7 +163,7 @@ __device__ __forceinline__ StepResult env_transition(const maze_env_batch& b, in
         } else {
             out.reward = __ldg(luts.revisit + cnt);   // :194
         }
-        visit_store(vp, (unsigned)((st.epoch << 8) | (cnt < 255 ? cnt + 1 : 255)), pol);   // :196
+        pol_store(vp, (unsigned)((st.epoch << 8) | (cnt < 255 ? cnt + 1 : 255)), pol);   // :196
         visit_bit_set(b, e, nr, nc);
         st.r = nr;
         st.c = nc;

@@ -4,14 +4,10 @@
 #pragma once
 #include "maze_common.cuh"
 
-#ifndef MAZE_FIELD_THREADS
-#define MAZE_FIELD_THREADS 128
-#endif
-#ifndef MAZE_METRIC_THREADS
-#define MAZE_METRIC_THREADS 384   /* 128 .. 512 measured on B200: 384 = 3 CTAs x 12 warps per SM is the best for maze_difficulty */
-#endif
-constexpr int FIELD_THREADS = MAZE_FIELD_THREADS;     // maze_fields / toroidal fields kernels (block BFS: barrier-bound)
-constexpr int METRIC_THREADS = MAZE_METRIC_THREADS;   // maze_difficulty and the scored generation kernel (latency-bound pointer walks)
+constexpr int FIELD_THREADS = 128;    // maze_fields / toroidal fields kernels (block BFS: barrier-bound)
+// maze_difficulty and the scored generation kernel (latency-bound pointer walks).  128 .. 512 measured on B200:
+// 384 = 3 CTAs x 12 warps per SM is the best for maze_difficulty.
+constexpr int METRIC_THREADS = 384;
 constexpr unsigned short DIST_INF = 0xffffu;
 
 struct FieldSmem {

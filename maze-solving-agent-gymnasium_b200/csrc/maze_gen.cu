@@ -28,19 +28,6 @@
 #include "maze_metrics.cuh"
 #include "maze_walls.cuh"
 
-#ifdef MAZE_GEN_PROFILE   // scratch instrumentation: cycles per phase, summed over mazes
-__device__ unsigned long long g_gen_prof[8];
-#define GEN_TICK(i) do { if ((threadIdx.x & 31) == 0) { long long _n = clock64(); atomicAdd(&g_gen_prof[i], (unsigned long long)(_n - _t)); _t = _n; } } while (0)
-extern "C" int maze_debug_gen_profile(unsigned long long* out, int reset) {
-    cudaDeviceSynchronize();
-    cudaMemcpyFromSymbol(out, g_gen_prof, sizeof(g_gen_prof));
-    if (reset) { unsigned long long z[8] = {0}; cudaMemcpyToSymbol(g_gen_prof, z, sizeof(z)); }
-    return 0;
-}
-#else
-#define GEN_TICK(i) do {} while (0)
-#endif
-
 namespace {
 
 constexpr int GEN_THREADS = METRIC_THREADS;   // CTA-per-maze kernel (scores with maze_metrics)
@@ -470,17 +457,12 @@ maze_generate_warp_kernel(GenParams p) {
             if (lane == 0) mm[MAZE_META_SOL_LEN] = -1;
             continue;
         }
-#ifdef MAZE_GEN_PROFILE
-        long long _t = clock64();
-#endif
         Walls w;
         int si, sj;
         generate_walls(w, (flags >> 8) & 0xff, nr, nc, p.seed,
                        (u64)(p.slot_id_base + m) | ((u64)(unsigned)gen_count << 40), (unsigned)p.candidate_base, si, sj);
-        GEN_TICK(1);
         const int goal = select_goal(w, si, sj);
         const int gi = goal >> 8, gj = goal & 0xff;
-        GEN_TICK(2);
         if (tor) {   // grid + start / goal now, fields by maze_fields_toroidal_kernel (block-level BFS on the torus)
             write_stripped_grid(w, Hb, Wb, gi, gj, p.grids + (size_t)m * p.slot);
             __syncwarp();
@@ -494,7 +476,6 @@ maze_generate_warp_kernel(GenParams p) {
         }
         GoalField g;
         goal_field(w, gi, gj, si, sj, 2 * (H < W ? H : W), g);
-        GEN_TICK(5);
         encode_bordered(w, g, H, W, gi, gj, p.table + (size_t)m * p.slot, p.grids ? p.grids + (size_t)m * p.slot : nullptr);
         __syncwarp();
         if (lane == 0) {
@@ -505,7 +486,6 @@ maze_generate_warp_kernel(GenParams p) {
             mm[MAZE_META_MAX_STEPS] = max_steps_budget(H, W, sol_len);
             mm[MAZE_META_SPARE] = gen_count + 1;
         }
-        GEN_TICK(6);
     }
 }
 
@@ -607,9 +587,6 @@ maze_generate_kernel(GenParams p) {
             continue;
         }
 
-#ifdef MAZE_GEN_PROFILE
-        long long _t = clock64();
-#endif
         // Candidates are DRAWN four at a time, one per warp (the carving loop is a dependent chain that
         // leaves a lone warp mostly idle), and SCORED one after the other in candidate order by the CTA.
         constexpr int NW = GEN_THREADS / 32;
@@ -632,7 +609,6 @@ maze_generate_kernel(GenParams p) {
                     goal = select_goal(w, si, sj);
                 }
             }
-            GEN_TICK(1);
             for (int k = 0; k < NW && base + k < p.candidates; ++k) {
                 const int cand = base + k;
                 __syncthreads();   // previous item / candidate fully consumed before smem is reused
@@ -652,7 +628,6 @@ maze_generate_kernel(GenParams p) {
                     if (kScored) cell_bfs_distances(w, si, sj, f.dist, Wb);   // block distances from start for the metrics
                 }
                 __syncthreads();
-                GEN_TICK(2);
                 if constexpr (kScored) {
                     // McClendon difficulty of the bordered maze (base_maze_env.py:86-92; for border-less
                     // mazes lib/maze_generation.py:51), on block distances from start
@@ -664,7 +639,6 @@ maze_generate_kernel(GenParams p) {
                     __syncthreads();
                     if (p.candidates > 1 && s_take)
                         for (int i = tid; i < Hb * Wb; i += GEN_THREADS) keep[i] = f.grid[i];
-                    GEN_TICK(3);
                 }
             }
         }
@@ -686,9 +660,7 @@ maze_generate_kernel(GenParams p) {
             sr -= 1; sc -= 1; gr -= 1; gc -= 1;
         }
 
-        GEN_TICK(4);
         block_bfs(f, H, W, tor, gr * W + gc);
-        GEN_TICK(5);
         encode_step_table(f, H, W, tor, gr, gc, p.table + (size_t)m * p.slot);
         if (p.grids) {
             uint8_t* g = p.grids + (size_t)m * p.slot;
@@ -704,7 +676,6 @@ maze_generate_kernel(GenParams p) {
             mm[MAZE_META_SPARE] = gen_count + 1;
             if (kScored && p.difficulty) p.difficulty[item] = s_keep_diff;
         }
-        GEN_TICK(6);
     }
 }
 

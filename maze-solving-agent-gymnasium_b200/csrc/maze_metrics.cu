@@ -5,15 +5,6 @@
 #include "maze_metrics.cuh"
 #include "maze_walls.cuh"
 
-#ifdef MAZE_METRICS_PROFILE
-extern "C" int maze_debug_metrics_profile(unsigned long long* out, int reset) {
-    cudaDeviceSynchronize();
-    cudaMemcpyFromSymbol(out, g_met_prof, sizeof(g_met_prof));
-    if (reset) { unsigned long long z[12] = {0}; cudaMemcpyToSymbol(g_met_prof, z, sizeof(z)); }
-    return 0;
-}
-#endif
-
 namespace {
 
 __global__ void __launch_bounds__(METRIC_THREADS)
@@ -41,9 +32,6 @@ maze_difficulty_kernel(const uint8_t* __restrict__ grids, const int32_t* __restr
         __syncthreads();
         const int start_idx = ((start & 0xffff) + pad) * Wb + (start >> 16) + pad;
         const int goal_idx = ((goal & 0xffff) + pad) * Wb + (goal >> 16) + pad;
-#ifdef MAZE_METRICS_PROFILE
-        long long _mt = clock64();
-#endif
         // block distances from start: bit-parallel BFS over the cell lattice by warp 0 (one level per
         // cell distance, whatever the frontier size); lattices above 64 x 64 cells use the CTA-wide BFS
         const int nr = (Hb - 1) / 2, nc = (Wb - 1) / 2;
@@ -59,7 +47,6 @@ maze_difficulty_kernel(const uint8_t* __restrict__ grids, const int32_t* __restr
         } else {
             block_bfs(f, Hb, Wb, false, start_idx);
         }
-        MET_TICK(0);
         maze_metrics(f, ms, Hb, Wb, start_idx, goal_idx, s_out, true, ext_out != nullptr);
         if (ext_out && tid < MAZE_METRIC_EXT_WORDS) ext_out[(size_t)item * MAZE_METRIC_EXT_WORDS + tid] = s_out.ext[tid];
         if (tid == 0) {

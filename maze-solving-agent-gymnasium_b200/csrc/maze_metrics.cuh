@@ -64,13 +64,6 @@ __device__ __forceinline__ bool atomic_min_u16(unsigned short* p, unsigned short
     }
 }
 
-#ifdef MAZE_METRICS_PROFILE
-static __device__ unsigned long long g_met_prof[12];
-#define MET_TICK(i) do { __syncthreads(); if (threadIdx.x == 0) { long long _n = clock64(); atomicAdd(&g_met_prof[i], (unsigned long long)(_n - _mt)); _mt = _n; } } while (0)
-#else
-#define MET_TICK(i) do {} while (0)
-#endif
-
 struct MazeMetrics {
     double difficulty, complexity, L, DE, D;
     int sol_len, de_count;
@@ -103,9 +96,6 @@ __device__ inline void maze_metrics(const FieldSmem& f, const MetricsSmem& ms, i
         return;
     }
     const int sol_len = (int)f.dist[goal_idx] + 1;
-#ifdef MAZE_METRICS_PROFILE
-    long long _mt = clock64();
-#endif
 
     // ---- 1. per-cell neighbour count / turn / node flags
     for (int ci = tid; ci < cells; ci += nthr) {
@@ -141,7 +131,6 @@ __device__ inline void maze_metrics(const FieldSmem& f, const MetricsSmem& ms, i
         if ((tid & 31) == 0) atomicAdd(&s_open, open);
     }
 
-    MET_TICK(1);
     // ---- 2. mark the solution (goal -> start along BFS parents); D = decision cells on it
     if (tid == 0) {
         int b = goal_idx, dcount = 0, junctions = 0, crossings = 0, turns = 0, arrived = 0;
@@ -163,7 +152,6 @@ __device__ inline void maze_metrics(const FieldSmem& f, const MetricsSmem& ms, i
     }
     __syncthreads();
 
-    MET_TICK(2);
     // ---- 3. parent node and edge length of every node (walk straight up to the next node)
     for (int ci = tid; ci < cells; ci += nthr) {
         if (!(ms.flags[ci] & MF_NODE) || ci == start_c) continue;
@@ -182,7 +170,6 @@ __device__ inline void maze_metrics(const FieldSmem& f, const MetricsSmem& ms, i
     }
     __syncthreads();
 
-    MET_TICK(3);
     auto is_sol = [&](int ci) { return (ms.flags[ci] & MF_SOL) != 0; };
     auto nbof = [&](int ci) { return ms.flags[ci] & MF_NB; };
     auto is_plain = [&](int ci) { return !is_sol(ci) && nbof(ci) != 3; };
@@ -209,7 +196,6 @@ __device__ inline void maze_metrics(const FieldSmem& f, const MetricsSmem& ms, i
             jup[ci] = (unsigned short)y;
         }
         __syncthreads();
-        MET_TICK(9);
         const int gr = goal_idx / Wb, gc = goal_idx % Wb;
         for (int de = tid; de < cells; de += nthr) {
             if (!is_dead_end_off(de)) continue;
@@ -253,7 +239,6 @@ __device__ inline void maze_metrics(const FieldSmem& f, const MetricsSmem& ms, i
             }
         }
         __syncthreads();
-        MET_TICK(10);
         // 4c.  The reference walks the dead ends in row-major order: dead end d counts unless a decision point of
         // its chain was recorded by an earlier counted dead end, and a counted dead end records the first decision
         // point of its chain.  With rec[P] = smallest index of a counted dead end whose first decision point is P,
@@ -331,7 +316,6 @@ __device__ inline void maze_metrics(const FieldSmem& f, const MetricsSmem& ms, i
         __syncthreads();
     }
 
-    MET_TICK(4);
     // ---- 5. smallest dead-end rank below every off-solution node (adjacency order of the reference)
     for (int ci = tid; ci < cells; ci += nthr) {
         if (!is_dead_end_off(ci)) continue;
@@ -345,7 +329,6 @@ __device__ inline void maze_metrics(const FieldSmem& f, const MetricsSmem& ms, i
             y = ms.pnode[y];
         }
     }
-    MET_TICK(5);
     // ---- 6. component root of every plain node
     for (int ci = tid; ci < cells; ci += nthr) {
         if (!(ms.flags[ci] & MF_NODE) || !is_plain(ci)) continue;
@@ -355,7 +338,6 @@ __device__ inline void maze_metrics(const FieldSmem& f, const MetricsSmem& ms, i
     }
     __syncthreads();
 
-    MET_TICK(6);
     // ---- 7. every tree edge goes to at most one hallway (maze_complexity_evaluation.py:186-221)
     for (int n = tid; n < cells; n += nthr) {
         if (!(ms.flags[n] & MF_NODE) || n == start_c) continue;
@@ -381,7 +363,6 @@ __device__ inline void maze_metrics(const FieldSmem& f, const MetricsSmem& ms, i
     }
     __syncthreads();
 
-    MET_TICK(7);
     // ---- 8. hallway complexity -> branch (maze_complexity_evaluation.py:223-259,286-308)
     for (int r = tid; r < cells; r += nthr) {
         if (!(ms.flags[r] & MF_NODE) || ms.comp[r] != r) continue;
@@ -397,7 +378,6 @@ __device__ inline void maze_metrics(const FieldSmem& f, const MetricsSmem& ms, i
     }
     __syncthreads();
 
-    MET_TICK(8);
     // ---- 9. reduce: sum and product over branches
     double tsum = 0.0, tprod = 1.0;
     for (int k = tid; k < cells; k += nthr) {

@@ -26,9 +26,7 @@ constexpr int WIN_CELLS = WIN * WIN;
 constexpr int WIN_ENVS = OBS_THREADS / 16;
 constexpr int WIN_FLOATS = 3 * WIN_CELLS;
 
-#ifndef MAZE_WIN_MINB
-#define MAZE_WIN_MINB 4
-#endif
+constexpr int WIN_MIN_BLOCKS = 4;   // __launch_bounds__ of both window kernels
 
 // masks of one window row -> the row's 3 x 15 output bytes in shared memory
 __device__ __forceinline__ void window_row_to_smem(uint8_t* sl, unsigned m0, unsigned m1, unsigned m2) {
@@ -64,7 +62,7 @@ __device__ __forceinline__ void window_stream_out(const uint8_t* s_out, float* _
     }
 }
 
-__global__ void __launch_bounds__(OBS_THREADS, MAZE_WIN_MINB)
+__global__ void __launch_bounds__(OBS_THREADS, WIN_MIN_BLOCKS)
 maze_window_kernel(maze_env_batch b, float* __restrict__ window, double* __restrict__ agent_norm,
                    double* __restrict__ target_norm) {
     __shared__ __align__(16) uint8_t s_out[WIN_ENVS * WIN_FLOATS];
@@ -89,7 +87,7 @@ maze_window_kernel(maze_env_batch b, float* __restrict__ window, double* __restr
 constexpr int WINB_PER = 2;   // 4 measured slower (4.7 vs 5.2 TB/s at 262 144 envs: fewer CTAs per SM by shared memory)
 constexpr int WINB_ENVS = WIN_ENVS * WINB_PER;
 
-__global__ void __launch_bounds__(OBS_THREADS, MAZE_WIN_MINB)
+__global__ void __launch_bounds__(OBS_THREADS, WIN_MIN_BLOCKS)
 maze_window_bordered_kernel(maze_env_batch b, float* __restrict__ window, double* __restrict__ agent_norm,
                             double* __restrict__ target_norm) {
     __shared__ __align__(16) uint8_t s_out[WINB_ENVS * WIN_FLOATS];

@@ -10,12 +10,7 @@
 namespace {
 
 constexpr int STEP_THREADS = 256;
-#ifndef MAZE_STEP_MINB1
-#define MAZE_STEP_MINB1 6
-#endif
-#ifndef MAZE_STEP_MINB2
-#define MAZE_STEP_MINB2 5
-#endif
+constexpr int STEP_MIN_BLOCKS_EPT1 = 6, STEP_MIN_BLOCKS_EPT2 = 5;   // __launch_bounds__ of maze_step_kernel
 
 // EPT environments per thread (env = base + k * STEP_THREADS keeps every access coalesced): the
 // loads of all EPT envs are issued phase by phase before anything waits on them.  The dependent
@@ -23,11 +18,11 @@ constexpr int STEP_THREADS = 256;
 // counter is only fetched when the move is legal (a wall hit needs no counter), which matters
 // because every such fetch costs a whole DRAM line.
 template <int EPT, bool kStats, bool kTiled>
-__global__ void __launch_bounds__(STEP_THREADS, EPT == 2 ? MAZE_STEP_MINB2 : MAZE_STEP_MINB1)
+__global__ void __launch_bounds__(STEP_THREADS, EPT == 2 ? STEP_MIN_BLOCKS_EPT2 : STEP_MIN_BLOCKS_EPT1)
 maze_step_kernel(maze_env_batch b, const uint8_t* __restrict__ actions, uint32_t mode, StepLuts luts) {
     const int base = blockIdx.x * (STEP_THREADS * EPT) + threadIdx.x;
 
-    const uint64_t pol_state = l2_policy<MAZE_STATE_POLICY>(), pol_table = l2_policy<MAZE_TABLE_POLICY>();
+    const uint64_t pol_state = l2_policy(), pol_table = l2_policy();
     // ---- phase 1: per-env words
     uint64_t raw[EPT];
     int m[EPT], a[EPT];
@@ -37,8 +32,8 @@ maze_step_kernel(maze_env_batch b, const uint8_t* __restrict__ actions, uint32_t
         const int e = base + k * STEP_THREADS;
         valid[k] = e < b.num_envs;
         const int ee = valid[k] ? e : b.num_envs - 1;
-        raw[k] = pol_load<MAZE_STATE_POLICY>(reinterpret_cast<const unsigned long long*>(b.state) + ee, pol_state);
-        m[k] = pol_load<MAZE_STATE_POLICY>(b.env_maze + ee, pol_state);
+        raw[k] = pol_load(reinterpret_cast<const unsigned long long*>(b.state) + ee, pol_state);
+        m[k] = pol_load(b.env_maze + ee, pol_state);
         a[k] = __ldcs(actions + ee) & 3;
     }
 
@@ -52,7 +47,7 @@ maze_step_kernel(maze_env_batch b, const uint8_t* __restrict__ actions, uint32_t
         if (do_reset[k] && (mode & MAZE_STEP_WIN_NEXT) && (flags & MAZE_ST_WON)) {
             m[k] += b.pool_stride;
             if (m[k] >= b.num_mazes) m[k] -= b.num_mazes;
-            pol_store<MAZE_STATE_POLICY>(b.env_maze + base + k * STEP_THREADS, m[k], pol_state);
+            pol_store(b.env_maze + base + k * STEP_THREADS, m[k], pol_state);
         }
         const int2 shape = __ldg(reinterpret_cast<const int2*>(b.meta + (size_t)m[k] * MAZE_META_WORDS));
         hw[k] = shape.x | (shape.y << 16);
@@ -86,24 +81,18 @@ maze_step_kernel(maze_env_batch b, const uint8_t* __restrict__ actions, uint32_t
         npos[k] = nr | (nc << 16);
         idx[k] = nr * W + nc;
         vidx[k] = kTiled ? ((((nr >> 2) * ((W + 3) >> 2) + (nc >> 2)) << 4) | ((nr & 3) << 2) | (nc & 3)) : idx[k];
-#ifdef MAZE_EXP_NOTABLE
-        tb[k] = 1 | ((idx[k] & 3) << 1) | ((idx[k] & 3) << 4);
-#else
-        tb[k] = pol_load_nc<MAZE_TABLE_POLICY>(b.table + (size_t)m[k] * b.slot + idx[k], pol_table);
-#endif
+        tb[k] = pol_load_nc(b.table + (size_t)m[k] * b.slot + idx[k], pol_table);
     }
 
     // ---- phase 4: visit counter, only for legal moves
-    const uint64_t pol = l2_policy<MAZE_VISIT_POLICY>();
+    const uint64_t pol = l2_policy();
     uint32_t vis[EPT];
     bool moved[EPT];
 #pragma unroll
     for (int k = 0; k < EPT; ++k) {
         moved[k] = valid[k] && !do_reset[k] && inb[k] && (tb[k] & MAZE_TAB_OPEN);
         vis[k] = 0;
-#ifndef MAZE_EXP_NOVISIT
-        if (moved[k]) vis[k] = visit_load(VISIT_AT(b, base + k * STEP_THREADS, vidx[k]), pol);
-#endif
+        if (moved[k]) vis[k] = pol_load(VISIT_AT(b, base + k * STEP_THREADS, vidx[k]), pol);
     }
 
     // ---- phase 5: transition + outputs
@@ -139,10 +128,8 @@ maze_step_kernel(maze_env_batch b, const uint8_t* __restrict__ actions, uint32_t
                     reward = __ldg(luts.revisit + cnt);   // :194
                     rcode = MAZE_REC_REWARD(MAZE_REC_KIND_REVISIT, (uint32_t)cnt);
                 }
-#ifndef MAZE_EXP_NOVISIT
-                visit_store(VISIT_AT(b, e, vidx[k]), (unsigned)((st.epoch << 8) | (cnt < 255 ? cnt + 1 : 255)), pol);   // :196
+                pol_store(VISIT_AT(b, e, vidx[k]), (unsigned)((st.epoch << 8) | (cnt < 255 ? cnt + 1 : 255)), pol);   // :196
                 visit_bit_set(b, e, npos[k] & 0xffff, npos[k] >> 16);
-#endif
                 st.r = npos[k] & 0xffff;
                 st.c = npos[k] >> 16;
                 st.tab = tb[k];
@@ -175,7 +162,7 @@ maze_step_kernel(maze_env_batch b, const uint8_t* __restrict__ actions, uint32_t
 
         if (!valid[k]) continue;
 
-        pol_store<MAZE_STATE_POLICY>(reinterpret_cast<unsigned long long*>(b.state) + e, (unsigned long long)pack_state(st), pol_state);
+        pol_store(reinterpret_cast<unsigned long long*>(b.state) + e, (unsigned long long)pack_state(st), pol_state);
         // `target` only changes when the env's maze does: the restart after a win (next pool maze, or the
         // regenerated slot).  The buffer persists between steps, so it is rewritten only then, and
         // target_dirty tells a host mirror that this launch touched it.

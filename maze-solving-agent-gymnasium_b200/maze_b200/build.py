@@ -8,7 +8,8 @@ import subprocess
 PKG_ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REPO_ROOT = os.path.dirname(PKG_ROOT)
 CSRC = os.path.join(PKG_ROOT, "csrc")
-# MAZE_B200_LIB: load an alternative build of the same ABI (A/B experiments); default in-tree .so
+# MAZE_B200_LIB: load another build of the same ABI (e.g. one written with build(out=...), to compare two
+# builds); default in-tree .so
 LIB_PATH = os.environ.get("MAZE_B200_LIB") or os.path.join(PKG_ROOT, "libmaze_b200.so")
 INCLUDE = os.path.join(REPO_ROOT, "include")
 
@@ -25,13 +26,13 @@ def needs_build() -> bool:
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build(force: bool = False, verbose: bool = False, defines=(), out=None) -> str:
+def build(force: bool = False, verbose: bool = False, out=None) -> str:
     if out is None and not force and not needs_build():
         return LIB_PATH
     nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
     cmd = [nvcc, "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
            "--compiler-options", "-fPIC", "-shared", "-I", INCLUDE, "-I", CSRC, "-o", out or LIB_PATH]
-    cmd += [f"-D{d}" for d in defines] + sources()
+    cmd += sources()
     if verbose:
         cmd.insert(1, "-Xptxas=-v")
     res = subprocess.run(cmd, capture_output=True, text=True)

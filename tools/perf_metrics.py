@@ -1,23 +1,15 @@
-"""Scratch: maze_difficulty throughput and per-phase cycles (library built with -DMAZE_METRICS_PROFILE)."""
-import ctypes, os, sys
+"""Scratch: maze_difficulty throughput per generation algorithm."""
+import os, sys
 import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "maze-solving-agent-gymnasium_b200"))
 import maze_b200 as mb
 M = int(sys.argv[1]) if len(sys.argv) > 1 else 32768
-lib = mb.cabi.lib()
-prof = getattr(lib, "maze_debug_metrics_profile", None)
 for algo in ("r-prim", "dfs", "prim&kill"):
     pool = mb.MazePool(M, (81, 81)); pool.generate(algorithms=algo, seed=3)
     pool.difficulty(); torch.cuda.synchronize()
-    buf = (ctypes.c_ulonglong * 12)()
-    if prof: prof(buf, 1)
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
     ev[0].record(); pool.difficulty(); pool.difficulty(); ev[1].record(); torch.cuda.synchronize()
     ms = ev[0].elapsed_time(ev[1]) / 2
-    line = f"{algo:10s} M={M}: {ms:.2f} ms  {M/ms*1e3:.3e} mazes/s"
-    if prof:
-        prof(buf, 1); tot = sum(buf) or 1
-        line += "  phases% bfs/init/sol/parents/DE/minleaf/comp/edges/branch: " + " ".join(f"{100*x/tot:.0f}" for x in list(buf)[:9]) + "  DE split 4a/4b/4c: " + " ".join(f"{100*x/tot:.0f}" for x in (buf[9], buf[10], buf[4])) + f"  kcyc/maze {tot/2/M/1e3:.0f}"
-    print(line, flush=True)
+    print(f"{algo:10s} M={M}: {ms:.2f} ms  {M/ms*1e3:.3e} mazes/s", flush=True)
     del pool
