@@ -16,6 +16,8 @@ Modules
   env_port.py    PortEnv: step/reset exactly as the reference computes them (A* per step);
                  ClosedFormEnv: the O(1) table-driven restatement the kernels implement
   generation.py  r-prim / dfs / prim&kill generators + goal selection + validity checks
+  gen_stream.py  bit-exact model of the device generators' random stream (Philox-keyed PCG32)
+  gen_exact.py   exact generator output distributions on small lattices, best-of-k, chi-square
   metrics.py     McClendon difficulty/complexity, Kim-Crawfis L / D / DE and the unused
                  Kim-Crawfis metrics (density, T, J, CR, AC/FDE/BDE, L_DE, *_sharp)
   qlearn.py      tabular Q / double-Q update rules
