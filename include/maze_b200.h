@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define MAZE_ABI_VERSION 12
+#define MAZE_ABI_VERSION 13
 
 /* argument errors */
 #define MAZE_E_NULL   (-1) /* required pointer is NULL                        */
@@ -203,9 +203,11 @@ int maze_step_decode_host(const uint32_t* records, int64_t n, const int32_t* sha
 /* Measurement aid, not part of the env path (tools/perf_scatter_rmw.py, DESIGN.md section 4.1): one launch that
  * streams maze_step's coalesced words for every env of `b` (streams != 0) and lets rmw_per_1024 of every 1024 envs do
  * one 2-byte read-modify-write in arr (uint16 [n_elems]) -- pattern 0: uniform random element; 1: cell-major
- * cell * B + env with a random cell per env; 2: as 1 with one cell per warp.  Overwrites b's outputs and state. */
+ * cell * B + env with a random cell per env; 2: as 1 with one cell per warp.  Pattern 1 sends retouch_per_1024 of
+ * every 1024 envs that did an RMW in launch - 1 back to that launch's cell.  order 1 runs the CTAs in reverse on odd
+ * launches, as maze_step does; hints 0..3 pick the L2 policies (csrc/maze_bench.cu).  Overwrites b's outputs and state. */
 int maze_bench_scatter_rmw(maze_ctx* ctx, const maze_env_batch* b, const uint8_t* actions, uint16_t* arr, int64_t n_elems, int pattern,
-                           int rmw_per_1024, uint32_t launch, int streams, void* stream);
+                           int rmw_per_1024, uint32_t launch, int streams, int order, int retouch_per_1024, int hints, void* stream);
 
 /* k_steps consecutive transitions per env in one call, for action sequences known in advance
  * (scripted / random exploration, replaying tapes): exactly the result of k_steps maze_step calls

@@ -22,6 +22,7 @@ struct maze_ctx {
     void*  d_scratch;       // library-owned scratch (candidate wall planes of scored generation), grown on demand
     size_t scratch_bytes;
     void*  net_profile;     // maze_net.cu: in-situ launch timing (events), created on first use
+    unsigned step_launches; // maze_step calls so far: odd ones run the CTAs in reverse order
     char   err[512];
 };
 

@@ -33,7 +33,9 @@ inline StepLuts step_luts(const maze_ctx* ctx) {
 //   action, obs, reward, flags   written / read once               -> always streaming (.cs)
 // The first three are all loaded and stored L2 evict_last.  The default policy and evict_first
 // measured within 2 % of it on B200, except evict_first on the visit sectors, which was 20 %
-// slower: the store misses the sector its own load fetched (DESIGN.md §4.1).
+// slower: the store misses the sector its own load fetched (DESIGN.md §4.1).  With maze_step's CTA order
+// reversed on every other launch, evict_first on state / env_maze and no hint on the visits were 1 % and
+// 2.7 % slower than evict_last.
 __device__ __forceinline__ uint64_t l2_policy() {
     uint64_t p;
     asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));

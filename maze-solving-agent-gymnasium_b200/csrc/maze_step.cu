@@ -4,6 +4,10 @@
 // (coalesced 8-byte load/store); the maze is read through its one-byte-per-block step table
 // (L2/L1 resident for a maze pool); the only scattered DRAM access is the 2-byte visit counter of
 // the block stepped onto, fetched only for legal moves, from a cell-major array.
+// Every other maze_step launch runs its CTAs in reverse order, so the envs stepped last in one launch
+// are stepped first in the next, while their state word, maze id and the visit counters they just
+// wrote may still be in L2.  Each env's transition reads only its own data, so the order cannot
+// change a result.
 // Reference semantics: gymnasium_env/envs/base_maze_env.py:136-210, lib/maze_view.py:165-197.
 #include "maze_env.cuh"
 
@@ -19,8 +23,9 @@ constexpr int STEP_MIN_BLOCKS_EPT1 = 6, STEP_MIN_BLOCKS_EPT2 = 5;   // __launch_
 // because every such fetch costs a whole DRAM line.
 template <int EPT, bool kStats, bool kTiled>
 __global__ void __launch_bounds__(STEP_THREADS, EPT == 2 ? STEP_MIN_BLOCKS_EPT2 : STEP_MIN_BLOCKS_EPT1)
-maze_step_kernel(maze_env_batch b, const uint8_t* __restrict__ actions, uint32_t mode, StepLuts luts) {
-    const int base = blockIdx.x * (STEP_THREADS * EPT) + threadIdx.x;
+maze_step_kernel(maze_env_batch b, const uint8_t* __restrict__ actions, uint32_t mode, StepLuts luts, bool reverse) {
+    const int blk = reverse ? (int)(gridDim.x - 1 - blockIdx.x) : (int)blockIdx.x;
+    const int base = blk * (STEP_THREADS * EPT) + threadIdx.x;
 
     const uint64_t pol_state = l2_policy(), pol_table = l2_policy();
     // ---- phase 1: per-env words
@@ -356,7 +361,8 @@ extern "C" int maze_step(maze_ctx* ctx, const maze_env_batch* b, const uint8_t* 
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int ept = b->num_envs < 64 * 1024 ? 1 : 2;   // small batches: more CTAs beats more loads per thread
     auto grid_for = [&](int e) { return (b->num_envs + STEP_THREADS * e - 1) / (STEP_THREADS * e); };
-    auto launch = [&](auto kernel, int e) { kernel<<<grid_for(e), STEP_THREADS, 0, st>>>(*b, actions, mode, luts); };
+    const bool reverse = (ctx->step_launches++ & 1) != 0;
+    auto launch = [&](auto kernel, int e) { kernel<<<grid_for(e), STEP_THREADS, 0, st>>>(*b, actions, mode, luts, reverse); };
 #define MAZE_STEP_DISPATCH(EPT_)                                                                          \
     do {                                                                                                  \
         if (stats) { if (tiled) launch(maze_step_kernel<EPT_, true, true>, EPT_); else launch(maze_step_kernel<EPT_, true, false>, EPT_); } \

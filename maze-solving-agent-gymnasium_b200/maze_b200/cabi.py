@@ -6,7 +6,7 @@ import os
 
 from .build import LIB_PATH
 
-ABI_VERSION = 12
+ABI_VERSION = 13
 BATCH_BORDERED = 1
 
 # constants mirrored from include/maze_b200.h
@@ -108,7 +108,7 @@ SIGNATURES = {
     "maze_step": (C.c_int, [C.c_void_p, C.POINTER(MazeEnvBatch), C.c_void_p, C.c_uint32, C.c_void_p]),
     "maze_step_decode_host": (C.c_int, [C.c_void_p, C.c_int64] + [C.c_void_p] * 7),
     "maze_bench_scatter_rmw": (C.c_int, [C.c_void_p, C.POINTER(MazeEnvBatch), C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_uint32,
-                                         C.c_int, C.c_void_p]),
+                                         C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "maze_step_many": (C.c_int, [C.c_void_p, C.POINTER(MazeEnvBatch), C.c_void_p, C.c_int, C.c_uint32, C.POINTER(MazeStepTrace),
                                  C.c_int, C.c_void_p]),
     "maze_reset": (C.c_int, [C.c_void_p, C.POINTER(MazeEnvBatch), C.c_void_p, C.c_void_p]),

@@ -6,7 +6,13 @@ mazes, a [slot, B] uint16 visit array of 54 GB -- for every combination of {stre
 {uniform, cell-major per env, cell-major per warp}, and the real maze_step kernel at steady state beside them.
 Writes gpurun_out/scatter_rmw.json (copy the summary into profiles/).
 
+--order times the CTA order instead: streams + cell-major RMW with the CTAs in the same order every launch
+("fwd") against reversed on odd launches ("alt", what maze_step does), with and without lag-1 re-touches (a
+share of the touched atoms that the same env touched one launch earlier: 0.20 in a count of the bench's random
+walk), under the L2-policy variants of csrc/maze_bench.cu.  Writes its summary to --out.
+
     python tools/perf_scatter_rmw.py [--envs 4096000] [--iters 200] [--once PATTERN STREAMS]   # --once: one config, for ncu
+    python tools/perf_scatter_rmw.py --order [--rounds 3] [--out scatter_order.json]
 """
 from __future__ import annotations
 
@@ -30,6 +36,9 @@ def main():
     ap.add_argument("--mazes", type=int, default=1000)
     ap.add_argument("--iters", type=int, default=200)
     ap.add_argument("--once", nargs=2, type=int, default=None)
+    ap.add_argument("--order", action="store_true")
+    ap.add_argument("--rounds", type=int, default=3)
+    ap.add_argument("--out", default="scatter_order.json", help="--order: file the summary is written to")
     args = ap.parse_args()
     dev = torch.device("cuda:0")
     B = args.envs
@@ -41,8 +50,9 @@ def main():
     arr, n_elems = b.visits, b.visits.numel()
     stream = cabi.current_stream(dev)
 
-    def launch(pattern, rate, it, streams):
-        rc = lib.maze_bench_scatter_rmw(ctx.handle, C.byref(b._c), cabi.ptr(acts[it % 64]), cabi.ptr(arr), n_elems, pattern, rate, it, streams, stream)
+    def launch(pattern, rate, it, streams, order=0, retouch=0, hints=0):
+        rc = lib.maze_bench_scatter_rmw(ctx.handle, C.byref(b._c), cabi.ptr(acts[it % 64]), cabi.ptr(arr), n_elems, pattern, rate, it, streams,
+                                        order, retouch, hints, stream)
         ctx.check(rc, "maze_bench_scatter_rmw")
 
     def timed(fn, iters):
@@ -62,6 +72,8 @@ def main():
             launch(pattern, 410, i, streams)
         torch.cuda.synchronize()
         return
+    if args.order:
+        return order_study(args, b, acts, launch, timed)
     out = {"envs": B, "array_bytes": n_elems * 2, "rmw_fraction": 410 / 1024}
     # the real kernel at steady state (autoreset on, same maze pool): what the patterns are compared with
     mode = cabi.STEP_AUTORESET
@@ -83,6 +95,50 @@ def main():
     print(json.dumps(out, indent=1))
     os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
     json.dump(out, open(os.path.join(ROOT, "gpurun_out", "scatter_rmw.json"), "w"), indent=1)
+
+
+HINTS = {1: "all_evict_last", 2: "state_evict_first_visits_evict_last", 3: "state_evict_last_visits_default"}
+
+
+def order_study(args, b, acts, launch, timed):
+    import statistics
+    mode = cabi.STEP_AUTORESET
+    for i in range(300):
+        b.step(acts[i % 64], mode)
+    state_keep = b.state.clone()
+    configs = []
+    for rate in (410, 530):                       # the r02 assumption; 0.518 legal moves per env-step in the walk count
+        for lag1 in (0.0, 0.20):                  # share of touched atoms last touched one launch earlier
+            retouch = min(1024, round(lag1 * 1024 * 1024 / rate))   # of the envs whose previous launch did an RMW
+            for hints in HINTS:
+                for order in (0, 1):
+                    configs.append((rate, lag1, retouch, hints, order))
+    times = {c: [] for c in configs}
+    step_us = []
+    for _ in range(args.rounds):                  # rounds interleave the configs, so drift hits all of them alike
+        for c in configs:
+            rate, _, retouch, hints, order = c
+            times[c].append(timed(lambda i: launch(1, rate, i, 1, order, retouch, hints), args.iters))
+        b.state.copy_(state_keep)
+        step_us.append(timed(lambda i: b.step(acts[i % 64], mode), args.iters))
+    b.state.copy_(state_keep)
+    props = torch.cuda.get_device_properties(0)
+    out = {"envs": b.num_envs, "iters": args.iters, "rounds": args.rounds, "device": props.name,
+           "what": "median us per launch of streams + cell-major RMW (maze_bench_scatter_rmw pattern 1); fwd = same CTA order every launch, "
+                   "alt = reversed on odd launches",
+           "maze_step_us_this_build": statistics.median(step_us), "variants": []}
+    for rate in (410, 530):
+        for lag1 in (0.0, 0.20):
+            for hints, hname in HINTS.items():
+                fwd, alt = (statistics.median(times[c]) for c in configs if c[0] == rate and c[1] == lag1 and c[3] == hints)
+                retouch = next(c[2] for c in configs if c[0] == rate and c[1] == lag1)
+                out["variants"].append({"rmw_per_1024": rate, "lag1_share": lag1, "retouch_per_1024": retouch, "hints": hname,
+                                        "fwd_us": fwd, "alt_us": alt, "alt_over_fwd": alt / fwd,
+                                        "fwd_runs_us": times[(rate, lag1, retouch, hints, 0)], "alt_runs_us": times[(rate, lag1, retouch, hints, 1)]})
+    print(json.dumps(out, indent=1))
+    if os.path.dirname(args.out):
+        os.makedirs(os.path.dirname(args.out), exist_ok=True)
+    json.dump(out, open(args.out, "w"), indent=1)
 
 
 if __name__ == "__main__":
