@@ -45,7 +45,6 @@ struct GenParams {
     int smem_hw;
     int smem_cells;          // 0 when no metrics are needed
     int candidates;          // best-of-k by McClendon difficulty (base_maze_env.py:78-97); 1 = raw generator
-    int candidate_base;      // test hook (MAZE_GEN_CANDIDATE_BASE): RNG key of candidate c is candidate_base + c
     int only_toroidal;       // CTA kernel: skip bordered slots (the warp kernel did them)
     int* work_counter;       // warp kernel: next unclaimed item (mazes differ in cost: claim dynamically)
     double* difficulty;      // [n] optional out: difficulty of the maze kept for item k
@@ -461,7 +460,7 @@ maze_generate_warp_kernel(GenParams p) {
         Walls w;
         int si, sj;
         generate_walls(w, (flags >> 8) & 0xff, nr, nc, p.seed,
-                       (u64)(p.slot_id_base + m) | ((u64)(unsigned)gen_count << 40), (unsigned)p.candidate_base, si, sj);
+                       (u64)(p.slot_id_base + m) | ((u64)(unsigned)gen_count << 40), 0u, si, sj);
         const int goal = select_goal(w, si, sj);
         const int gi = goal >> 8, gj = goal & 0xff;
         if (tor) {   // grid + start / goal now, fields by maze_fields_toroidal_kernel (block-level BFS on the torus)
@@ -513,7 +512,7 @@ maze_generate_planes_kernel(GenParams p) {
         Walls w;
         int si, sj;
         generate_walls(w, (flags >> 8) & 0xff, nr, nc, p.seed,
-                       (u64)(p.slot_id_base + m) | ((u64)(unsigned)mm[MAZE_META_SPARE] << 40), (unsigned)(p.candidate_base + cand), si, sj);
+                       (u64)(p.slot_id_base + m) | ((u64)(unsigned)mm[MAZE_META_SPARE] << 40), (unsigned)cand, si, sj);
         const int goal = select_goal(w, si, sj);
         unsigned long long* out = p.planes + (size_t)work * PLANE_WORDS;
         out[lane] = w.e.a0; out[32 + lane] = w.e.a1;
@@ -606,7 +605,7 @@ maze_generate_kernel(GenParams p) {
                     goal = (int)in[2 * MAZE_GEN_MAX_CELLS + 1];
                 } else {
                     generate_walls(w, algo, nr, nc, p.seed, (u64)(p.slot_id_base + m) | ((u64)(unsigned)gen_count << 40),
-                                   (unsigned)(p.candidate_base + base + wid), si, sj);
+                                   (unsigned)(base + wid), si, sj);
                     goal = select_goal(w, si, sj);
                 }
             }
@@ -703,10 +702,6 @@ extern "C" int maze_generate(maze_ctx* ctx, uint8_t* grids, int32_t* meta, uint8
     const bool scored = candidates > 1 || difficulty != nullptr;
     p.smem_cells = scored ? ((max_h + 1) / 2) * ((max_w + 1) / 2) : 0;
     p.candidates = candidates;
-    // Test hook: draw candidates b .. b + k - 1 of every slot instead of 0 .. k - 1, so that a test can materialise each
-    // candidate of a best-of-k selection on its own (candidates = 1) and re-score it with the oracle.
-    const char* cb = getenv("MAZE_GEN_CANDIDATE_BASE");
-    p.candidate_base = cb ? atoi(cb) : 0;
     p.only_toroidal = scored ? 0 : 1;
     p.difficulty = difficulty;
     p.work_counter = nullptr;
@@ -748,7 +743,7 @@ extern "C" int maze_generate(maze_ctx* ctx, uint8_t* grids, int32_t* meta, uint8
     // into library-owned scratch, chunk by chunk, and the CTA kernel only scores and keeps.  Regeneration queues
     // (device-side count, a few slots per step) stay on the single-kernel path.
     constexpr int CHUNK = 8192;
-    if (scored && candidates > 1 && !count_dev && n >= 16 && !getenv("MAZE_GEN_SINGLE_KERNEL")) {
+    if (scored && candidates > 1 && !count_dev && n >= 16) {
         const int chunk = n < CHUNK ? n : CHUNK;
         const size_t need = (size_t)chunk * candidates * PLANE_WORDS * sizeof(unsigned long long);
         if (ctx->scratch_bytes < need) {

@@ -2,8 +2,8 @@
 //
 // maze_window: one warp per env writes the float32 [3, 15, 15] crop around the agent
 // (lib/maze_handler.py:4-99) -- 2 700 B of coalesced streaming stores per env; the maze comes from
-// the L2-resident step table, the visit counters from the env-major visit array (a window row is
-// 30 contiguous bytes).  HBM-write bound.
+// the L2-resident step table, the visited state from the env's visit bitmap or visit counters.
+// HBM-write bound.
 // maze_direction_mask: one thread per env, four table bytes (lib/maze_handler.py:122-162,
 // simple_maze_env.py:41-50, toroidal_maze_env.py:57-70).
 #include "maze_env.cuh"

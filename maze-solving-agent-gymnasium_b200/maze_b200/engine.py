@@ -226,12 +226,11 @@ class MazeBatch:
     def __init__(self, pool: MazePool, num_envs: int, env_maze=None, stats: bool = False, pool_stride: int = 1,
                  queue: bool = False, visit_layout: str = "cell", visit_bits: bool = False):
         """visit_layout: "cell" = [slot, B] (best for the -v0 step: envs sharing a block share lines),
-        "env" = [B, slot] (best when the 15x15 window is read every step: rows are contiguous),
         "tile" = env-major with 4x4 block tiles per 32-byte sector (a walking agent stays in a sector).
         visit_bits: also keep the one-bit-per-block "visited this episode" map (1 KB per env at 81 x 81) that the -v1
         window and the replay encode read their non_visited channel from."""
-        if visit_layout not in ("cell", "env", "tile"):
-            raise ValueError("visit_layout must be 'cell', 'env' or 'tile'")
+        if visit_layout not in ("cell", "tile"):
+            raise ValueError("visit_layout must be 'cell' or 'tile'")
         self.visit_layout = visit_layout
         self.pool = pool
         self.device = pool.device

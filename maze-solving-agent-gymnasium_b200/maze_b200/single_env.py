@@ -51,7 +51,7 @@ class BaseMazeEnv(Env):
             seed = random.getrandbits(62)   # the reference draws from the global `random`, so seeding it seeds us
         self._seed = int(seed)
         self._pool = MazePool(1, pool_shape, self.device)
-        self._batch = MazeBatch(self._pool, 1, visit_layout="env" if self.ENRICH else "cell")
+        self._batch = MazeBatch(self._pool, 1, visit_layout="tile" if self.ENRICH else "cell")
         self._act = torch.zeros(1, dtype=torch.uint8, device=self.device)
         self._difficulty = torch.zeros(1, dtype=torch.float64, device=self.device)
         self.action_space = spaces.Discrete(4)

@@ -19,8 +19,6 @@ from __future__ import annotations
 from types import SimpleNamespace
 from typing import Optional
 
-import os
-
 import numpy as np
 import torch
 
@@ -80,12 +78,12 @@ class MazeVectorEnv(_VectorBase):
         (variable-size envs: START_SHAPE and +(4, 4), simple_variable_maze_env.py:17,97);
         `algorithm_schedule` = ((wins, algorithm), ...) switches a slot's generator by its win count
         (off_policy_trainer.py:302-310: ((5, "prim&kill"), (10, "dfs"))).
-        regenerate_ahead (on_win="regenerate", with or without a curriculum; default 3, MAZE_REGEN_AHEAD=0 turns it off): keep
+        regenerate_ahead (on_win="regenerate", with or without a curriculum; None = the default, 3; 0 turns it off): keep
         the next k mazes of every slot in a shadow ring that a side stream refills, so that a win costs a 13 KB copy
         instead of the generator's latency (include/maze_b200.h: maze_regen_swap).  Same mazes either way; k x 13 KB per slot.
         visit_layout: "cell" (default; best for one launch per step), "tile" (env-major in 4 x 4 block tiles:
         best for the fused multi-step paths -- step_many, the Q-learning rollout -- and the default with
-        enrich, where the 15 x 15 window then reads <= 25 whole sectors per env), "env" (env-major rows)."""
+        enrich, where the 15 x 15 window then reads <= 25 whole sectors per env)."""
         if topology not in ("euclid", "toroidal"):
             raise ValueError("topology must be 'euclid' or 'toroidal'")
         if on_win not in ("keep", "next", "regenerate"):
@@ -126,7 +124,7 @@ class MazeVectorEnv(_VectorBase):
             raise ValueError("grow / algorithm_schedule act when a maze is regenerated: use on_win='regenerate'")
         self.wins = torch.zeros(pool.num_mazes, dtype=torch.int32, device=self.device)
         if regenerate_ahead is None:
-            regenerate_ahead = int(os.environ.get("MAZE_REGEN_AHEAD", "3") or 0)
+            regenerate_ahead = 3
         self.regenerate_depth = min(8, int(regenerate_ahead))   # True -> 1
         self.regenerate_ahead = self.regenerate_depth > 0 and on_win == "regenerate"
         self._ahead = None   # built on the first drain (and again after load_state_dict)

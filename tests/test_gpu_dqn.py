@@ -21,7 +21,7 @@ def _setup(B_per_maze=4, visit_bits=False):
                                   [m["toroidal"] for m in mazes])
     B = B_per_maze * len(mazes)
     env_maze = np.arange(B) % len(mazes)
-    batch = mb.MazeBatch(pool, B, env_maze=torch.from_numpy(env_maze.astype(np.int32)).cuda(), visit_layout="env", visit_bits=visit_bits)
+    batch = mb.MazeBatch(pool, B, env_maze=torch.from_numpy(env_maze.astype(np.int32)).cuda(), visit_layout="cell", visit_bits=visit_bits)
     envs = [ClosedFormEnv(mazes[k]["grid"], mazes[k]["start"], mazes[k]["goal"], mazes[k]["toroidal"], enrich=True) for k in env_maze]
     return mb, batch, envs
 

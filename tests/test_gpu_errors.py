@@ -62,6 +62,8 @@ def test_host_side_validation():
     with pytest.raises(ValueError):
         mb.MazeBatch(pool, 4, visit_layout="diagonal")
     with pytest.raises(ValueError):
+        mb.MazeBatch(pool, 4, visit_layout="env")
+    with pytest.raises(ValueError):
         mb.MazeVectorEnv(8, shape=(21, 21), on_win="regenerate", num_mazes=4)     # needs one slot per env
     with pytest.raises(ValueError):
         mb.MazeVectorEnv(8, shape=(11, 11), enrich=True)                          # no 15x15 window in an 11x11 maze

@@ -120,30 +120,24 @@ def test_best_of_k_selection(algo, toroidal):
 
 
 @pytest.mark.parametrize("algo,toroidal", [("r-prim", False), ("dfs", False), ("prim&kill", False), ("r-prim", True)])
-def test_best_of_six_keeps_the_reference_winner(algo, toroidal, monkeypatch):
+def test_best_of_six_keeps_the_reference_winner(algo, toroidal):
     """generate_maze (base_maze_env.py:78-97, toroidal_maze_env.py:40-54): of the six draws the FIRST minimum of the
-    McClendon difficulty is kept (scores equal to 1e-12 relative are one minimum: oracle.gen_exact.best_candidate).  Every candidate is materialised on its own (the MAZE_GEN_CANDIDATE_BASE test hook
-    shifts the RNG key, candidates = 1), re-scored with the ORACLE (oracle.metrics.mcclendon, itself pinned to the
-    reference's values), and the oracle's winner must be the maze the best-of-six launch kept -- through both code paths:
-    the bulk pipeline (planes kernel + scoring kernel) and the single-kernel path of the regeneration queue."""
+    McClendon difficulty is kept (scores equal to 1e-12 relative are one minimum: oracle.gen_exact.best_candidate).  Every candidate is
+    drawn on its own by the bit-exact stream model (oracle.gen_stream.stream_maze, candidate c of slot m), re-scored with the
+    ORACLE (oracle.metrics.mcclendon, itself pinned to the reference's values), and the oracle's winner must be the maze the
+    best-of-six launch kept -- through both code paths: the bulk pipeline (planes kernel + scoring kernel) and the
+    single-kernel path of the regeneration queue."""
     import maze_b200 as mb
     from oracle.gen_exact import best_candidate
+    from oracle.gen_stream import stream_maze
     from oracle.metrics import mcclendon
     n, S = 40, 21
-    cands = []
-    for c in range(6):
-        monkeypatch.setenv("MAZE_GEN_CANDIDATE_BASE", str(c))
-        pool = mb.MazePool(n, (S, S))
-        pool.generate(algorithms=algo, toroidal=toroidal, seed=99)
-        meta = pool.meta_host()
-        cands.append([(pool.grid_host(m).copy(), int(meta[m, 2]), int(meta[m, 3])) for m in range(n)])
-    monkeypatch.delenv("MAZE_GEN_CANDIDATE_BASE")
+    cands = [[stream_maze(algo, (S, S), toroidal, 99, m, 0, c) for m in range(n)] for c in range(6)]
 
-    def oracle_score(grid, start, goal):
-        s, g = (start & 0xffff, start >> 16), (goal & 0xffff, goal >> 16)
+    def oracle_score(start, goal, grid):
         if toroidal:   # scored on the bordered maze before stripping (lib/maze_generation.py:48-56)
-            grid, s, g = np.pad(grid, 1), (s[0] + 1, s[1] + 1), (g[0] + 1, g[1] + 1)
-        return mcclendon(grid, s, g)[0]
+            grid, start, goal = np.pad(grid, 1), (start[0] + 1, start[1] + 1), (goal[0] + 1, goal[1] + 1)
+        return mcclendon(grid, start, goal)[0]
 
     winners = []
     for m in range(n):
@@ -162,7 +156,7 @@ def test_best_of_six_keeps_the_reference_winner(algo, toroidal, monkeypatch):
     for m in range(n):
         best, scores = winners[m]
         for pool in (bulk, queue):
-            np.testing.assert_array_equal(pool.grid_host(m), cands[best][m][0], err_msg=f"slot {m}: kept maze is not candidate {best} {scores}")
+            np.testing.assert_array_equal(pool.grid_host(m), cands[best][m][2], err_msg=f"slot {m}: kept maze is not candidate {best} {scores}")
         assert dout[m].item() == pytest.approx(scores[best], rel=1e-9)
 
 
@@ -234,26 +228,23 @@ def test_metrics_calculator_mirror_exposes_the_unused_methods():
 
 
 @pytest.mark.parametrize("toroidal", [False, True])
-def test_bulk_best_of_k_pipeline_equals_the_single_kernel_path(toroidal, monkeypatch):
+def test_bulk_best_of_k_pipeline_equals_the_single_kernel_path(toroidal):
     """Bulk best-of-k draws its candidates with the warp generator into scratch and scores them in the CTA
-    kernel; the regeneration-queue path does both in one kernel.  Same candidates, same scores, same kept maze."""
+    kernel; the regeneration-queue path (device-side count) does both in one kernel.  Same candidates, same scores,
+    same kept maze."""
     import maze_b200 as mb
     n, shape = 300, (41, 41)
     algos = ["r-prim", "dfs", "prim&kill"] * 100
-
-    def run():
-        pool = mb.MazePool(n, shape)
-        d = torch.full((n,), float("nan"), dtype=torch.float64, device="cuda")
-        pool.generate(algorithms=algos, toroidal=toroidal, seed=21, candidates=6, difficulty_out=d)
-        return pool, d
-    two, d2 = run()
-    monkeypatch.setenv("MAZE_GEN_SINGLE_KERNEL", "1")
-    one, d1 = run()
-    monkeypatch.delenv("MAZE_GEN_SINGLE_KERNEL")
+    ids, count = torch.arange(n, dtype=torch.int32, device="cuda"), torch.tensor([n], dtype=torch.int32, device="cuda")
+    two, one = mb.MazePool(n, shape), mb.MazePool(n, shape)
+    d2, d1 = (torch.full((n,), float("nan"), dtype=torch.float64, device="cuda") for _ in range(2))
+    two.generate(algorithms=algos, toroidal=toroidal, seed=21, candidates=6, difficulty_out=d2)
+    one.generate(algorithms=algos, toroidal=toroidal, seed=21)                                   # configure the slots, generation count 1 ...
+    one.meta[:, mb.cabi.META_SPARE] = 0                                                          # ... back to 0: same RNG keys as `two`
+    one.generate(ids=ids, count_dev=count, configure=False, seed=21, candidates=6, difficulty_out=d1)   # the single-kernel path
     assert torch.equal(two.grids, one.grids) and torch.equal(two.table, one.table) and torch.equal(two.meta, one.meta)
     np.testing.assert_allclose(d2.cpu().numpy(), d1.cpu().numpy(), rtol=1e-12)
     # a second generation of the same slots (generation count 1) differs from the first and again agrees
     two.generate(algorithms=algos, toroidal=toroidal, seed=21, candidates=6)
-    monkeypatch.setenv("MAZE_GEN_SINGLE_KERNEL", "1")
-    one.generate(algorithms=algos, toroidal=toroidal, seed=21, candidates=6)
+    one.generate(ids=ids, count_dev=count, configure=False, seed=21, candidates=6)
     assert torch.equal(two.grids, one.grids) and torch.equal(two.meta, one.meta)

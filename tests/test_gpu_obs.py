@@ -30,7 +30,7 @@ def _replay(meta, z, visit_layout, on_step, visit_bits=False):
 
 
 @pytest.mark.parametrize("name", ["steps", "steps81"])
-@pytest.mark.parametrize("visit_layout", ["env", "cell", "tile", "cell+bits", "tile+bits"])
+@pytest.mark.parametrize("visit_layout", ["cell", "tile", "cell+bits", "tile+bits"])
 def test_window_matches_reference_traces(name, visit_layout):
     """"+bits": the non_visited channel comes from the one-bit-per-block visited map (maze_env_batch.visit_bits, the -v1
     default of MazeVectorEnv) instead of the visit counters."""
@@ -90,7 +90,7 @@ def test_window_against_oracle_with_autoreset(visit_bits):
     pool = mb.MazePool.from_grids([m["grid"] for m in mazes], [m["start"] for m in mazes], [m["goal"] for m in mazes],
                                   [m["toroidal"] for m in mazes])
     B = len(mazes)
-    batch = mb.MazeBatch(pool, B, visit_layout="env", visit_bits=visit_bits)
+    batch = mb.MazeBatch(pool, B, visit_layout="cell", visit_bits=visit_bits)
     envs = [ClosedFormEnv(m["grid"], m["start"], m["goal"], m["toroidal"], enrich=True) for m in mazes]
     batch.reset()
     obs = [e.reset()[0] for e in envs]

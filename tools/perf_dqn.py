@@ -12,7 +12,7 @@ def timed(fn, reps):
     for _ in range(reps): fn()
     e[1].record(); torch.cuda.synchronize()
     return e[0].elapsed_time(e[1]) / reps * 1e-3
-for lay in ("tile", "env"):
+for lay in ("tile", "cell"):
     B = 1048576
     venv = mb.MazeVectorEnv(B, shape=(81, 81), num_mazes=1000, enrich=True, seed=1234, on_win="next", stats=False, visit_layout=lay)
     venv.reset()

@@ -1,12 +1,12 @@
 """Scratch: maze_step time per launch for visit layouts x batch sizes, steady state, CUDA-graph replay.
-usage: python tools/perf_step.py [layouts] [sizes]   e.g.  cell,env,tile 1048576,4096000"""
+usage: python tools/perf_step.py [layouts] [sizes]   e.g.  cell,tile 1048576,4096000"""
 import os, sys
 import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "maze-solving-agent-gymnasium_b200"))
 import maze_b200 as mb
 
-layouts = (sys.argv[1] if len(sys.argv) > 1 else "cell,env,tile").split(",")
+layouts = (sys.argv[1] if len(sys.argv) > 1 else "cell,tile").split(",")
 sizes = [int(x) for x in (sys.argv[2] if len(sys.argv) > 2 else "1048576,4096000").split(",")]
 M, TAPE = 1000, 16
 S = int(sys.argv[3]) if len(sys.argv) > 3 else 81

@@ -4,7 +4,7 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "maze-solving-agent-gymnasium_b200"))
 import maze_b200 as mb
-for B, lay in ((262144, "env"), (1048576, "env"), (1048576, "tile")):
+for B, lay in ((262144, "cell"), (1048576, "cell"), (1048576, "tile")):
     venv = mb.MazeVectorEnv(B, shape=(81, 81), num_mazes=1000, enrich=True, seed=1234, on_win="next", stats=False, visit_layout=lay)
     venv.reset()
     acts = torch.randint(0, 4, (B,), dtype=torch.uint8, device="cuda")
