@@ -3,6 +3,7 @@
 GPUs of one box, gradients summed with one NCCL all-reduce per optimiser step.
 
     python examples/train_ddqn.py --envs 8192 --iters 200
+    python examples/train_ddqn.py --agent dqn --dropout 0.2      # the plain DQN target; Dropout(0.2) in the conv stage
     torchrun --nproc-per-node 8 --master-addr 127.0.0.1 examples/train_ddqn.py --envs 8192 --iters 200
 
 Everything runs in this repo's kernels: env step (maze_step), masked epsilon-greedy (maze_dqn_select), bit-packed replay
@@ -35,8 +36,12 @@ class DDQNLoop:
     """One rank's share of config 5."""
 
     def __init__(self, envs: int, batch: int, shape: int = 81, memory: int = 1 << 20, rank: int = 0, world: int = 1, device="cuda",
-                 lr: float = 1e-4, gamma: float = 0.9, target_every: int = 50, seed: int = 1, overlap: bool = True):
+                 lr: float = 1e-4, gamma: float = 0.9, target_every: int = 50, seed: int = 1, overlap: bool = True,
+                 agent: str = "ddqn", dropout: float = 0.0):
+        if agent not in ("ddqn", "dqn"):
+            raise ValueError(f"agent must be 'ddqn' or 'dqn', got {agent!r}")
         self.B, self.n, self.rank, self.world, self.overlap = envs, batch, rank, world, overlap
+        self.agent, self.dropout = agent, float(dropout)
         self.lr, self.gamma, self.target_every = lr, gamma, target_every
         self.device = torch.device(device)
         self.env = mb.MazeVectorEnv(envs, shape=(shape, shape), enrich=True, on_win="regenerate", algorithms="r-prim", seed=seed,
@@ -44,7 +49,9 @@ class DDQNLoop:
                                     algorithm_schedule=((5, "prim&kill"), (10, "dfs")))   # off_policy_trainer.py:302-310
         self.memory = DeviceReplay(self.env, max(memory, envs), seed=rank)
         self.actor = MaskedEpsilonGreedy(self.env, 0.9, 0.05, 2000, seed=7, env_id_base=rank * envs)
-        self.net = DQNNet(self.device, max_batch=max(envs, batch), seed=0)     # same initial weights on every rank
+        # same initial weights on every rank; each rank draws its own dropout masks
+        self.net = DQNNet(self.device, max_batch=max(envs, batch), seed=0, dropout=dropout, double_q=agent == "ddqn",
+                          dropout_seed=(int(seed) << 32) | rank)
         self.q = torch.zeros((envs, 4), dtype=torch.float32, device=self.device)
         self.iters = 0
         self.opt_steps = 0
@@ -80,8 +87,8 @@ class DDQNLoop:
             net.update_target()
 
     def flop_per_iteration(self):
-        """Forward on B envs; per optimiser step forward on 3 n samples and backward (2 x forward) on n."""
-        return FWD_FLOP * (self.B + 5 * self.n)
+        """Forward on B envs; per optimiser step forward on 3 n samples (DQN: 2 n) and backward (2 x forward) on n."""
+        return FWD_FLOP * (self.B + (5 if self.agent == "ddqn" else 4) * self.n)
 
 
 def main():
@@ -92,13 +99,16 @@ def main():
     ap.add_argument("--shape", type=int, default=81)
     ap.add_argument("--memory", type=int, default=1 << 20)
     ap.add_argument("--no-overlap", action="store_true", help="all-reduce the whole gradient after the backward pass (and time it)")
+    ap.add_argument("--agent", choices=["ddqn", "dqn"], default="ddqn", help="double-Q target (ddqn_agent.py) or max target (dqn_agent.py)")
+    ap.add_argument("--dropout", type=float, default=0.0, help="Dropout p after the conv's LeakyReLU (the reference's DDQN: 0.2)")
     args = ap.parse_args()
     rank, local, world = mb.dist.env_from_torchrun()
     torch.cuda.set_device(local)
     device = torch.device("cuda", local)
     if world > 1:
         dist.init_process_group("nccl", device_id=device)
-    loop = DDQNLoop(args.envs, args.batch, args.shape, args.memory, rank, world, device, overlap=not args.no_overlap)
+    loop = DDQNLoop(args.envs, args.batch, args.shape, args.memory, rank, world, device, overlap=not args.no_overlap, agent=args.agent,
+                    dropout=args.dropout)
     warmup = max(5, min(20, args.iters // 4))
     for _ in range(warmup):
         loop.iterate()
@@ -120,7 +130,7 @@ def main():
     stats = loop.env.episode_statistics(reduce=world > 1)
     if rank == 0:
         n_opt = loop.opt_steps - opt0
-        print(json.dumps({"env_steps_per_s": world * args.envs * args.iters / dt, "optimizer_steps_per_s": n_opt / dt,
+        print(json.dumps({"agent": args.agent, "dropout": args.dropout, "env_steps_per_s": world * args.envs * args.iters / dt, "optimizer_steps_per_s": n_opt / dt,
                           "samples_per_s": world * args.batch * n_opt / dt, "n_gpus": world, "envs_per_gpu": args.envs,
                           "batch_per_gpu": args.batch, "ms_per_iteration": dt / args.iters * 1e3,
                           "allreduce_share": ar_ms * 1e-3 / dt, "tflops_per_gpu": loop.flop_per_iteration() * args.iters / dt / 1e12,

@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define MAZE_ABI_VERSION 13
+#define MAZE_ABI_VERSION 14
 
 /* argument errors */
 #define MAZE_E_NULL   (-1) /* required pointer is NULL                        */
@@ -431,12 +431,26 @@ int maze_dqn_select(maze_ctx* ctx, const maze_env_batch* b, const float* q_value
 
 /* ---- DQN / DDQN network on the tensor cores (north star item 4; BASELINE.json configs[4]) ------------
  * The net of agents/ddqn_agent.py:18-52 (dqn_agent.py:19-57 is the same without Dropout):
- *   Conv2d(3, 32, 3, padding 1) + LeakyReLU + MaxPool2d(2, 2) on the 3 x 15 x 15 window -> 32 x 7 x 7 = 1568
+ *   Conv2d(3, 32, 3, padding 1) + LeakyReLU + Dropout(p) + MaxPool2d(2, 2) on the 3 x 15 x 15 window -> 32 x 7 x 7 = 1568
  *   cat(conv features, 6 state floats) -> Linear(1574, 1024) + LeakyReLU -> Linear(1024, 512) + ReLU -> Linear(512, 4)
- * and its update, ddqn_agent.py:113-152: q(s, a) of the source net, a* = argmax q_source(s', .),
- * y = r + gamma * q_target(s', a*), MSE loss (mean), elementwise gradient clamp to +-1, AdamW.
- * The reference's Dropout(p = 0.2) -- active in every forward because the nets are never put in eval() -- is
- * NOT applied (documented deviation: parity is against the same net with dropout off).
+ * and its update: update = 0 (ddqn_agent.py:113-152): q(s, a) of the source net, a* = argmax q_source(s', .),
+ * y = r + gamma * q_target(s', a*); update = 1 (the plain DQN target): y = r + gamma * max_a q_target(s', a), no source
+ * forward on s'.  Then MSE loss (mean), elementwise gradient clamp to +-1, AdamW.  Neither target masks terminal states.
+ *
+ * Dropout: p = maze_dqn_net.dropout (0 = none, the default; the reference's DDQN uses 0.2 and, never calling eval(), drops
+ * in every forward).  It applies in training mode (eval = 0) to every forward of maze_dqn_backward (each draws its own
+ * mask) and to maze_dqn_forward / maze_dqn_features; eval = 1 turns it off everywhere, like nn.Module.eval().
+ *   pooled = first maximum over the 2 x 2 candidates of  keep ? fp32(LeakyReLU(conv + bias) * s) : +0,  then bf16,
+ *   s = fp32(1 / (1 - p)) (1.25 at p = 0.2).  A dropped element is +0 (torch's x * 0 is -0 for a negative x; the two
+ *   compare equal, so only the sign of a pooled zero differs).
+ * The keep bit of an element is a pure function of (dropout_seed, draw, forward id, sample, element):
+ *   Philox4x32-10, key (dropout_seed lo, hi), counter (e / 8, sample index, draw lo 32 bits, forward id),
+ *   e = ((py * 7 + px) * 32 + channel) * 4 + 2 dy + dx over the 14 x 14 conv positions (2 py + dy, 2 px + dx) the pool
+ *   reads; the block's 16-bit draw k = e % 8 is bits 16 (k & 1) .. +15 of output word k / 2;
+ *   keep iff draw < round(65536 (1 - p))  (P(keep) = 0.800003 at p = 0.2).
+ *   Forward ids: 0 source net on s, 1 source net on s', 2 target net on s', 3 maze_dqn_forward / maze_dqn_features.
+ * A caller bumps `draw` between calls (the Python DQNNet does on every forward, features and backward call) so that
+ * each call draws fresh masks; equal seeds and equal call sequences give bit-identical results.
  *
  * Parameters live in ONE flat fp32 buffer per net (source `params`, target `target`), laid out as
  *   conv weight [32, 3, 3, 3] | conv bias [32] | fc1 weight [1024, 1600] | fc1 bias [1024] |
@@ -475,7 +489,13 @@ typedef struct maze_dqn_net {
     float*    loss;       /* [1] loss of the last maze_dqn_backward                     (training)   */
     int32_t   max_batch;  /* samples per call the workspace was sized for                           */
     int32_t   reserved;
-} maze_dqn_net;
+    float     dropout;    /* Dropout p in [0, 1); 0 = no dropout                                    */
+    int32_t   update;     /* 0 double-Q target (DDQN), 1 max target (DQN)                           */
+    int32_t   eval;       /* 0 training mode (dropout active, as in the reference), 1 evaluation    */
+    int32_t   reserved2;
+    uint64_t  dropout_seed;  /* Philox key of the dropout masks                                     */
+    uint64_t  draw;          /* call counter: its low 32 bits are a word of the mask counter        */
+} maze_dqn_net;              /* all-zero new fields: no dropout, double-Q (the behaviour of ABI 13) */
 
 int64_t maze_dqn_net_workspace_bytes(int max_batch);
 
@@ -489,7 +509,8 @@ int maze_dqn_forward(maze_ctx* ctx, const maze_dqn_net* net, int which, const fl
                      float* q_out, void* stream);
 
 /* The conv stage alone: X [n, MAZE_NET_IN] bf16 feature rows; pool_idx (optional, [n, 1568] uint8: bits 0-1 the
- * max-pool choice dy * 2 + dx, bit 2 pre-activation > 0).  Exposed for the parity tests. */
+ * max-pool choice dy * 2 + dx, bit 2 the winner's pre-activation > 0, bit 3 the winner was dropped -- always 0 without
+ * dropout).  Dropout as for forward id 3.  Exposed for the parity tests. */
 int maze_dqn_features(maze_ctx* ctx, const maze_dqn_net* net, int which, const float* vec, const uint32_t* win, int n,
                       uint16_t* X, uint8_t* pool_idx, void* stream);
 

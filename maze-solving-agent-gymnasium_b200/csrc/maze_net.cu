@@ -1,8 +1,10 @@
 // DQN / DDQN network on the B200 tensor cores (sm_100a): forward, double-Q target, backward and AdamW of
 // the net of agents/ddqn_agent.py:18-52 (conv 3->32 3x3 pad 1, LeakyReLU, MaxPool 2 -> 1568 (+6) -> 1024
 // -> 512 -> 4) and its update agents/ddqn_agent.py:113-152 (double-Q target, MSE, gradient clamp +-1, AdamW),
-// reading the replay ring's bit-packed windows directly (csrc/maze_dqn.cu).  Dropout (p = 0.2 in the
-// reference, active because the reference never calls eval()) is not applied: see DESIGN.md.
+// reading the replay ring's bit-packed windows directly (csrc/maze_dqn.cu).  The net's Dropout (p = 0.2 in the
+// reference, active because the reference never calls eval()) runs in the conv epilogue when maze_dqn_net.dropout > 0
+// (mask stream: include/maze_b200.h); maze_dqn_net.update = 1 swaps the double-Q target for the plain DQN max target of
+// agents/dqn_agent.py.
 //
 // Dense contractions run as tcgen05.mma (bf16 x bf16 -> fp32 in TMEM), operands staged by TMA:
 //   net_gemm_kernel   C[M,N] = A[M,K] . B[N,K]^T, both operands K-major bf16, 128 x BN x 64 tiles, SWIZZLE_128B,
@@ -561,10 +563,47 @@ net_conv_image_kernel(const float* __restrict__ conv_w, uint8_t* __restrict__ im
     }
 }
 
-template <bool SAVE_IDX>
-__global__ void __launch_bounds__(FEAT_THREADS)
+// Dropout(p) between the LeakyReLU and the max-pool.  The keep mask is a pure function of (seed, draw, forward id,
+// sample, element): Philox4x32-10 with key (seed lo, seed hi) and counter (element block, sample, draw lo, forward id);
+// elements e = ((py * 7 + px) * 32 + channel) * 4 + 2 dy + dx of the 14 x 14 positions the pool reads, eight per block
+// (16-bit draw k = e % 8 is bits 16 (k & 1) .. + 15 of word k / 2), kept iff draw < threshold.
+struct NetDropout {
+    uint32_t k0, k1;      // key: the dropout seed
+    uint32_t draw;        // counter word 2: low 32 bits of maze_dqn_net.draw
+    uint32_t fwd;         // counter word 3: 0 source on s, 1 source on s', 2 target on s', 3 maze_dqn_forward / _features
+    uint32_t threshold;   // round(65536 (1 - p)): P(keep) = threshold / 65536
+    float scale;          // fp32(1 / (1 - p))
+};
+
+// The 128 keep bits of one pooled cell (bit 4 channel + 2 dy + dx of keep[channel / 8]): 16 consecutive Philox blocks,
+// shifted in from the top one byte per block.  Not unrolled: sixteen interleaved blocks took 246 registers, which would
+// halve the kernel's four CTAs per SM.
+__device__ __forceinline__ void dropout_keep_bits(const NetDropout& d, int smp, int cell, uint32_t (&keep)[4]) {
+#pragma unroll 1
+    for (int j = 0; j < 16; ++j) {   // block 16 cell + j: channels 2 j and 2 j + 1, four pool candidates each
+        Philox ph;
+        ph.k0 = d.k0;
+        ph.k1 = d.k1;
+        ph.c0 = (uint32_t)(16 * cell + j);
+        ph.c1 = (uint32_t)smp;
+        ph.c2 = d.draw;
+        ph.c3 = d.fwd;
+        ph.refill();
+        const uint32_t o[4] = {ph.o0, ph.o1, ph.o2, ph.o3};
+        uint32_t bits = 0;
+#pragma unroll
+        for (int k = 0; k < 8; ++k) bits |= (((o[k >> 1] >> (16 * (k & 1))) & 0xffffu) < d.threshold ? 1u : 0u) << k;
+        keep[0] = (keep[0] >> 8) | (keep[1] << 24);
+        keep[1] = (keep[1] >> 8) | (keep[2] << 24);
+        keep[2] = (keep[2] >> 8) | (keep[3] << 24);
+        keep[3] = (keep[3] >> 8) | (bits << 24);
+    }
+}
+
+template <bool SAVE_IDX, bool DROPOUT>
+__global__ void __launch_bounds__(FEAT_THREADS, DROPOUT ? 4 : 0)   // dropout: 128 registers, no spills, so 4 CTAs per SM still fit (0: no bound)
 net_features_kernel(const float* __restrict__ vec, const uint32_t* __restrict__ win, int n, const uint4* __restrict__ conv_w_image,
-                    const float* __restrict__ conv_b, bf16* __restrict__ X, uint8_t* __restrict__ pool_idx) {
+                    const float* __restrict__ conv_b, bf16* __restrict__ X, uint8_t* __restrict__ pool_idx, const NetDropout drop) {
     __shared__ __align__(128) uint8_t sR[FEAT_R_BYTES];
     __shared__ __align__(128) uint8_t sW[FEAT_W_BYTES];
     __shared__ __align__(16) bf16 sfeat[2][NET_CONV_OUT];
@@ -636,6 +675,11 @@ net_features_kernel(const float* __restrict__ vec, const uint32_t* __restrict__ 
                 }
             tc::umma_commit(bar_a);
         }
+        [[maybe_unused]] uint32_t keep[4] = {0u, 0u, 0u, 0u};
+        if constexpr (DROPOUT) {   // the mask is drawn while the MMAs run
+            const int py = (warp & 1) * 4 + (lane >> 3), px = lane & 7;
+            if (s0 + (warp >> 1) < n && py < 7 && px < 7) dropout_keep_bits(drop, s0 + (warp >> 1), py * 7 + px, keep);
+        }
         tc::mbar_wait(bar_a, phase);
         phase ^= 1u;
         tc::tc_fence_after();
@@ -643,7 +687,46 @@ net_features_kernel(const float* __restrict__ vec, const uint32_t* __restrict__ 
         //      lane / 8, px = lane % 8.  2 x 2 max-pool over the four class blocks (first maximum in scan order wins), bias,
         //      LeakyReLU.
         const int half = warp >> 1;
-        if (s0 + half < n) {
+        if constexpr (DROPOUT) {
+            // Dropout sits between the LeakyReLU and the pool, so every candidate is activated and masked before the
+            // comparison: candidate = kept ? fp32(LeakyReLU(acc + bias) * scale) : +0 (a dropped candidate, value 0, can
+            // beat negative ones).  idx bit 2: the winner's pre-activation > 0; bit 3: the winner was dropped.
+            if (s0 + half < n) {
+                const int py = (warp & 1) * 4 + (lane >> 3), px = lane & 7;
+                float m[32];
+                uint32_t v[32];
+                [[maybe_unused]] uint32_t c1 = 0, c2 = 0, cpos = 0, cdrop = 0;   // bit ch: the winner's class bits, sign, dropped
+#pragma unroll
+                for (int cls = 0; cls < 4; ++cls) {
+                    tc::tmem_ld32(tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)cls * 32u, v);
+                    tc::tmem_ld_wait();
+#pragma unroll
+                    for (int ch = 0; ch < 32; ++ch) {
+                        const float x = __uint_as_float(v[ch]) + sbias[ch];
+                        const bool kept = (keep[ch >> 3] >> (((ch & 7) << 2) | cls)) & 1u;
+                        const float y = kept ? (x > 0.f ? x : LRELU_SLOPE * x) * drop.scale : 0.f;
+                        const bool take = cls == 0 || y > m[ch];
+                        m[ch] = take ? y : m[ch];
+                        if constexpr (SAVE_IDX) {
+                            const uint32_t bit = 1u << ch;
+                            if (cls & 1) c1 = take ? (c1 | bit) : c1; else c1 = take ? (c1 & ~bit) : c1;
+                            if (cls & 2) c2 = take ? (c2 | bit) : c2;
+                            cpos = take ? (x > 0.f ? (cpos | bit) : (cpos & ~bit)) : cpos;
+                            cdrop = take ? (kept ? (cdrop & ~bit) : (cdrop | bit)) : cdrop;
+                        }
+                    }
+                }
+                if (py < 7 && px < 7) {
+                    const int q = py * 7 + px;
+#pragma unroll
+                    for (int ch = 0; ch < 32; ++ch) {
+                        if constexpr (SAVE_IDX)
+                            sidx[half][ch * 49 + q] = (uint8_t)(((c1 >> ch) & 1u) | (((c2 >> ch) & 1u) << 1) | (((cpos >> ch) & 1u) << 2) | (((cdrop >> ch) & 1u) << 3));
+                        sfeat[half][ch * 49 + q] = __float2bfloat16(m[ch]);
+                    }
+                }
+            }
+        } else if (s0 + half < n) {
             const int py = (warp & 1) * 4 + (lane >> 3), px = lane & 7;
             const bool valid = py < 7 && px < 7;
             float m[32];
@@ -778,7 +861,10 @@ net_head_q_kernel(const bf16* __restrict__ h2, int n, const float* __restrict__ 
 
 // Loss and the gradient at the head (ddqn_agent.py:131-143): q(s, a) from the source net, a* = argmax_a' q_source(s', a'),
 // y = r + gamma * q_target(s', a*), loss = mean (q(s, a) - y)^2.  Writes dL/d(pre-ReLU h2) [n, 512] bf16 and accumulates the
-// fc3 gradients.
+// fc3 gradients.  UPDATE == UPDATE_MAX_TARGET: the DQN target y = r + gamma * max_a' q_target(s', a') (no source forward on
+// s': h2_sn is not read and may be null).
+enum { UPDATE_DOUBLE_Q = 0, UPDATE_MAX_TARGET = 1 };
+template <int UPDATE>
 __global__ void __launch_bounds__(HEAD_THREADS, 2)
 net_head_loss_kernel(const bf16* __restrict__ h2_s, const bf16* __restrict__ h2_sn, const bf16* __restrict__ h2_tn, int n,
                      const float* __restrict__ w3, const float* __restrict__ b3, const float* __restrict__ tw3, const float* __restrict__ tb3,
@@ -803,7 +889,7 @@ net_head_loss_kernel(const bf16* __restrict__ h2_s, const bf16* __restrict__ h2_
     float rew_next = 0.f;
     if (s < n) {
         head_load_raw(h2_s + (size_t)s * NET_H2, lane, ra);
-        head_load_raw(h2_sn + (size_t)s * NET_H2, lane, rb);
+        if constexpr (UPDATE == UPDATE_DOUBLE_Q) head_load_raw(h2_sn + (size_t)s * NET_H2, lane, rb);
         head_load_raw(h2_tn + (size_t)s * NET_H2, lane, rc);
         act_next = action[s] & 3;
         rew_next = reward[s];
@@ -823,14 +909,14 @@ net_head_loss_kernel(const bf16* __restrict__ h2_s, const bf16* __restrict__ h2_
     for (; s < n; s += stride) {
         float h[16], hn[16], ht[16];
         head_expand(ra, h);
-        head_expand(rb, hn);
+        if constexpr (UPDATE == UPDATE_DOUBLE_Q) head_expand(rb, hn);
         head_expand(rc, ht);
         const int act = act_next;
         const float rew = rew_next;
         if (s + stride < n) {
             const size_t t = (size_t)(s + stride);
             head_load_raw(h2_s + t * NET_H2, lane, ra);
-            head_load_raw(h2_sn + t * NET_H2, lane, rb);
+            if constexpr (UPDATE == UPDATE_DOUBLE_Q) head_load_raw(h2_sn + t * NET_H2, lane, rb);
             head_load_raw(h2_tn + t * NET_H2, lane, rc);
             act_next = action[t] & 3;
             rew_next = reward[t];
@@ -839,21 +925,24 @@ net_head_loss_kernel(const bf16* __restrict__ h2_s, const bf16* __restrict__ h2_
 #pragma unroll
         for (int a = 0; a < 4; ++a) {
             qs[a] = head_dot(h, sw + a * NET_H2, lane);
-            qn[a] = head_dot(hn, sw + a * NET_H2, lane);
+            if constexpr (UPDATE == UPDATE_DOUBLE_Q) qn[a] = head_dot(hn, sw + a * NET_H2, lane);
             qt[a] = head_dot(ht, stw + a * NET_H2, lane);
         }
 #pragma unroll
         for (int a = 0; a < 4; ++a) {   // twelve independent butterfly reductions, interleaved by the compiler
             qs[a] = warp_sum(qs[a]) + b3[a];
-            qn[a] = warp_sum(qn[a]) + b3[a];
+            if constexpr (UPDATE == UPDATE_DOUBLE_Q) qn[a] = warp_sum(qn[a]) + b3[a];
             qt[a] = warp_sum(qt[a]) + tb3[a];
         }
         int best = 0;   // .max(1)[1]: first maximum
+        if constexpr (UPDATE == UPDATE_DOUBLE_Q) {
 #pragma unroll
-        for (int a = 1; a < 4; ++a)
-            if (qn[a] > qn[best]) best = a;
+            for (int a = 1; a < 4; ++a)
+                if (qn[a] > qn[best]) best = a;
+        }
         const float qsa = act == 0 ? qs[0] : act == 1 ? qs[1] : act == 2 ? qs[2] : qs[3];
-        const float qtb = best == 0 ? qt[0] : best == 1 ? qt[1] : best == 2 ? qt[2] : qt[3];
+        const float qtb = UPDATE == UPDATE_MAX_TARGET ? fmaxf(fmaxf(qt[0], qt[1]), fmaxf(qt[2], qt[3]))   // .max(1)[0]
+                                                      : best == 0 ? qt[0] : best == 1 ? qt[1] : best == 2 ? qt[2] : qt[3];
         const float target = qtb * gamma + rew;
         const float d = qsa - target;
         const float gq = 2.f * d * inv_n;   // d mean((q - y)^2) / d q
@@ -942,9 +1031,12 @@ constexpr uint32_t CB_A_BYTES = 64 * 256 * 2, CB_B_BYTES = 32 * 256 * 2;
 constexpr size_t CB_SMEM = CB_A_BYTES + CB_B_BYTES + 128;   // 48 KB (+ 9 KB static staging): three CTAs per SM overlap each other's build / MMA phases
 constexpr int CB_B_UNITS = 27 * 28;                          // (tap, window row 0..13, half row)
 
+// DROPOUT: the pool winner's gradient passes the Dropout backward first (0 if idx bit 3 says it was dropped, else times
+// drop_scale), then the LeakyReLU backward -- autograd's order.
+template <bool DROPOUT>
 __global__ void __launch_bounds__(CB_THREADS, 3)
 net_conv_bwd_tc_kernel(const bf16* __restrict__ dX, const uint8_t* __restrict__ pool_idx, const uint32_t* __restrict__ win, int n,
-                       float* __restrict__ gconv_w, float* __restrict__ gconv_b) {
+                       float* __restrict__ gconv_w, float* __restrict__ gconv_b, float drop_scale) {
     extern __shared__ uint8_t smem_raw[];
     __shared__ uint64_t bar;
     __shared__ uint32_t tmem_slot;
@@ -1039,6 +1131,7 @@ net_conv_bwd_tc_kernel(const bf16* __restrict__ dX, const uint8_t* __restrict__ 
                     const int at = o * 49 + py * 7 + 4 * h + j;
                     b = s_i[buf][at];
                     float gv = __bfloat162float(s_g[buf][at]);
+                    if constexpr (DROPOUT) gv = (b & 8u) ? 0.f : gv * drop_scale;
                     if (!(b & 4u)) gv *= LRELU_SLOPE;
                     const uint32_t hb = (uint32_t)__bfloat16_as_ushort(__float2bfloat16(gv));
                     word = (b & 1u) ? hb << 16 : hb;       // columns 2 px and 2 px + 1 share a word
@@ -1228,7 +1321,23 @@ int check_net(maze_ctx* ctx, const maze_dqn_net* net, bool train) {
         return maze_fail_arg(ctx, MAZE_E_NULL, "net training pointer");
     if (((uintptr_t)net->params & 15) || ((uintptr_t)net->target & 15) || ((uintptr_t)net->workspace & 255))
         return maze_fail_arg(ctx, MAZE_E_ALIGN, "net params (16 bytes) / workspace (256 bytes)");
+    if (!(net->dropout >= 0.f && net->dropout < 1.f)) return maze_fail_arg(ctx, MAZE_E_RANGE, "net dropout (0 <= p < 1)");
+    if (net->update != 0 && net->update != 1) return maze_fail_arg(ctx, MAZE_E_RANGE, "net update (0 double-Q, 1 max target)");
+    if (net->eval != 0 && net->eval != 1) return maze_fail_arg(ctx, MAZE_E_RANGE, "net eval (0 training, 1 evaluation)");
     return 0;
+}
+
+// The Dropout of forward `fwd`, or null when the net has none (p = 0, or evaluation mode)
+const NetDropout* dropout_of(const maze_dqn_net* net, uint32_t fwd, NetDropout& d) {
+    if (!(net->dropout > 0.f) || net->eval) return nullptr;
+    const double keep = 1.0 - (double)net->dropout;
+    d.k0 = (uint32_t)net->dropout_seed;
+    d.k1 = (uint32_t)(net->dropout_seed >> 32);
+    d.draw = (uint32_t)net->draw;
+    d.fwd = fwd;
+    d.threshold = (uint32_t)floor(65536.0 * keep + 0.5);
+    d.scale = (float)(1.0 / keep);
+    return &d;
 }
 
 // Split-K factor of a weight-gradient GEMM (tiles x k-blocks, persistent over `sms` CTAs): the one that minimises
@@ -1277,13 +1386,16 @@ inline void prof_mark(maze_ctx* ctx, cudaStream_t st, const char* label) {
 }
 
 int features(maze_ctx* ctx, bool save_idx, const float* vec, const uint32_t* win, int n, const float* params, const uint8_t* conv_image, bf16* X,
-             uint8_t* idx, cudaStream_t st) {
+             uint8_t* idx, cudaStream_t st, const NetDropout* drop = nullptr) {
     const int pairs = (n + 1) / 2;   // two samples per iteration
     const int grid = pairs < ctx->num_sms * 4 ? pairs : ctx->num_sms * 4;   // 128 TMEM columns per CTA: four CTAs per SM
-    const auto kernel = save_idx ? net_features_kernel<true> : net_features_kernel<false>;
-    kernel<<<grid, FEAT_THREADS, 0, st>>>(vec, win, n, reinterpret_cast<const uint4*>(conv_image), params + MAZE_NET_OFF_CONV_B, X, idx);
+    const auto kernel = drop ? (save_idx ? net_features_kernel<true, true> : net_features_kernel<false, true>)
+                             : (save_idx ? net_features_kernel<true, false> : net_features_kernel<false, false>);
+    kernel<<<grid, FEAT_THREADS, 0, st>>>(vec, win, n, reinterpret_cast<const uint4*>(conv_image), params + MAZE_NET_OFF_CONV_B, X, idx,
+                                          drop ? *drop : NetDropout{});
     MAZE_CHECK(cudaGetLastError());
-    prof_mark(ctx, st, save_idx ? "features (conv + pool, saves argmax)" : "features (conv + pool)");
+    prof_mark(ctx, st, drop ? (save_idx ? "features (conv + dropout + pool, saves argmax)" : "features (conv + dropout + pool)")
+                            : (save_idx ? "features (conv + pool, saves argmax)" : "features (conv + pool)"));
     return 0;
 }
 
@@ -1349,9 +1461,10 @@ extern "C" int maze_dqn_features(maze_ctx* ctx, const maze_dqn_net* net, int whi
     if (int rc = check_net(ctx, net, false)) return rc;
     if (!vec || !win || !X) return maze_fail_arg(ctx, MAZE_E_NULL, "maze_dqn_features pointer");
     if (n < 1) return maze_fail_arg(ctx, MAZE_E_RANGE, "maze_dqn_features: n");
+    NetDropout d;
     return features(ctx, pool_idx != nullptr, vec, win, n, which ? net->target : net->params,
                     carve(net->workspace, net->max_batch).conv_image[which], reinterpret_cast<bf16*>(X), pool_idx,
-                    static_cast<cudaStream_t>(stream));
+                    static_cast<cudaStream_t>(stream), dropout_of(net, 3, d));
 }
 
 extern "C" int maze_dqn_forward(maze_ctx* ctx, const maze_dqn_net* net, int which, const float* vec, const uint32_t* win, int n, float* q_out,
@@ -1364,7 +1477,8 @@ extern "C" int maze_dqn_forward(maze_ctx* ctx, const maze_dqn_net* net, int whic
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const Workspace w = carve(net->workspace, net->max_batch);
     const float* p = which ? net->target : net->params;
-    if (int rc = features(ctx, false, vec, win, n, p, w.conv_image[which], w.X, nullptr, st)) return rc;
+    NetDropout d;
+    if (int rc = features(ctx, false, vec, win, n, p, w.conv_image[which], w.X, nullptr, st, dropout_of(net, 3, d))) return rc;
     if (int rc = mlp_forward(ctx, w.X, n, reinterpret_cast<const bf16*>(which ? net->tw1_bf16 : net->w1_bf16),
                              reinterpret_cast<const bf16*>(which ? net->tw2_bf16 : net->w2_bf16), p, w.h1, w.h2, st))
         return rc;
@@ -1390,23 +1504,30 @@ extern "C" int maze_dqn_backward(maze_ctx* ctx, const maze_dqn_net* net, const f
     const bf16 *w1t = reinterpret_cast<const bf16*>(net->w1t_bf16), *w2t = reinterpret_cast<const bf16*>(net->w2t_bf16);
     prof_reset(ctx, st);
     MAZE_CHECK(cudaMemsetAsync(net->loss, 0, sizeof(float), st));
-    // forward: source net on states and next states, target net on next states
+    // forward: source net on states and next states (double-Q only: the DQN target does not need it), target net on next
+    // states; with dropout each forward draws its own mask, and the saved pool choices are forward 0's
     bf16* Xt = w.dX;   // the target net has its own conv weights, so its own features; dX is free until the backward-data GEMM
     const bf16 *tw1b = reinterpret_cast<const bf16*>(net->tw1_bf16), *tw2b = reinterpret_cast<const bf16*>(net->tw2_bf16);
-    if (int rc = features(ctx, true, vec, win, n, p, w.conv_image[0], w.X, w.idx, st)) return rc;
+    const bool double_q = net->update == 0;
+    NetDropout d[3];
+    const NetDropout* drop0 = dropout_of(net, 0, d[0]);
+    if (int rc = features(ctx, true, vec, win, n, p, w.conv_image[0], w.X, w.idx, st, drop0)) return rc;
     if (int rc = mlp_forward(ctx, w.X, n, w1b, w2b, p, w.h1, w.h2, st)) return rc;
-    if (int rc = features(ctx, false, next_vec, next_win, n, p, w.conv_image[0], w.X + np * NET_IN, nullptr, st)) return rc;
-    if (int rc = mlp_forward(ctx, w.X + np * NET_IN, n, w1b, w2b, p, w.h1 + np * NET_H1, w.h2 + np * NET_H2, st)) return rc;
-    if (int rc = features(ctx, false, next_vec, next_win, n, net->target, w.conv_image[1], Xt, nullptr, st)) return rc;
+    if (double_q) {
+        if (int rc = features(ctx, false, next_vec, next_win, n, p, w.conv_image[0], w.X + np * NET_IN, nullptr, st, dropout_of(net, 1, d[1]))) return rc;
+        if (int rc = mlp_forward(ctx, w.X + np * NET_IN, n, w1b, w2b, p, w.h1 + np * NET_H1, w.h2 + np * NET_H2, st)) return rc;
+    }
+    if (int rc = features(ctx, false, next_vec, next_win, n, net->target, w.conv_image[1], Xt, nullptr, st, dropout_of(net, 2, d[2]))) return rc;
     if (int rc = mlp_forward(ctx, Xt, n, tw1b, tw2b, net->target, w.h1t_tn, w.h2_tn, st)) return rc;
     {
         const int grid = (n + 7) / 8 < 2 * ctx->num_sms ? (n + 7) / 8 : 2 * ctx->num_sms;   // two CTAs per SM; the fc3 gradient is merged with one atomic per CTA and entry
-        MAZE_CHECK(cudaFuncSetAttribute(net_head_loss_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)HEAD_LOSS_SMEM));
-        net_head_loss_kernel<<<grid, HEAD_THREADS, HEAD_LOSS_SMEM, st>>>(w.h2, w.h2 + np * NET_H2, w.h2_tn, n, p + MAZE_NET_OFF_W3, p + MAZE_NET_OFF_B3,
-                                                                         net->target + MAZE_NET_OFF_W3, net->target + MAZE_NET_OFF_B3, action, reward, gamma,
-                                                                         w.dh2, gr + MAZE_NET_OFF_W3, gr + MAZE_NET_OFF_B3, net->loss, qsa_out);
+        const auto head = double_q ? net_head_loss_kernel<UPDATE_DOUBLE_Q> : net_head_loss_kernel<UPDATE_MAX_TARGET>;
+        MAZE_CHECK(cudaFuncSetAttribute(head, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)HEAD_LOSS_SMEM));
+        head<<<grid, HEAD_THREADS, HEAD_LOSS_SMEM, st>>>(w.h2, double_q ? w.h2 + np * NET_H2 : nullptr, w.h2_tn, n, p + MAZE_NET_OFF_W3, p + MAZE_NET_OFF_B3,
+                                                         net->target + MAZE_NET_OFF_W3, net->target + MAZE_NET_OFF_B3, action, reward, gamma,
+                                                         w.dh2, gr + MAZE_NET_OFF_W3, gr + MAZE_NET_OFF_B3, net->loss, qsa_out);
         MAZE_CHECK(cudaGetLastError());
-        prof_mark(ctx, st, "head: Q, double-Q target, loss, dQ, fc3 gradients");
+        prof_mark(ctx, st, double_q ? "head: Q, double-Q target, loss, dQ, fc3 gradients" : "head: Q, max target, loss, dQ, fc3 gradients");
     }
     // fc2: dW2 = dh2^T . h1 (MN-major operands: straight from the [n, features] activations), db2 = colsum(dh2),
     //      dh1 = (dh2 . W2) * LeakyReLU'(h1)
@@ -1438,9 +1559,10 @@ extern "C" int maze_dqn_backward(maze_ctx* ctx, const maze_dqn_net* net, const f
     if (int rc = launch_gemm(ctx, EPI_BIAS_ACT, fc_tile(n), w.dh1, NET_H1, w1t, NET_H1, g, 1, st)) return rc;
     prof_mark(ctx, st, "fc1 backward-data GEMM");
     {
-        MAZE_CHECK(cudaFuncSetAttribute(net_conv_bwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CB_SMEM));
+        const auto conv_bwd = drop0 ? net_conv_bwd_tc_kernel<true> : net_conv_bwd_tc_kernel<false>;
+        MAZE_CHECK(cudaFuncSetAttribute(conv_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CB_SMEM));
         const int grid = n < ctx->num_sms * 3 ? n : ctx->num_sms * 3;   // 48 KB of operands + 9 KB of staging per CTA: three fit an SM
-        net_conv_bwd_tc_kernel<<<grid, CB_THREADS, CB_SMEM, st>>>(w.dX, w.idx, win, n, gr + MAZE_NET_OFF_CONV_W, gr + MAZE_NET_OFF_CONV_B);
+        conv_bwd<<<grid, CB_THREADS, CB_SMEM, st>>>(w.dX, w.idx, win, n, gr + MAZE_NET_OFF_CONV_W, gr + MAZE_NET_OFF_CONV_B, drop0 ? drop0->scale : 1.f);
         MAZE_CHECK(cudaGetLastError());
     }
     prof_mark(ctx, st, "conv gradient (un-pool + implicit GEMM)");

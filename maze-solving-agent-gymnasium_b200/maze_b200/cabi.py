@@ -6,7 +6,7 @@ import os
 
 from .build import LIB_PATH
 
-ABI_VERSION = 13
+ABI_VERSION = 14
 BATCH_BORDERED = 1
 
 # constants mirrored from include/maze_b200.h
@@ -77,7 +77,8 @@ class MazeDqnNet(C.Structure):
     _fields_ = [("params", C.c_void_p), ("target", C.c_void_p), ("grads", C.c_void_p), ("adam_m", C.c_void_p), ("adam_v", C.c_void_p),
                 ("w1_bf16", C.c_void_p), ("w2_bf16", C.c_void_p), ("w1t_bf16", C.c_void_p), ("w2t_bf16", C.c_void_p),
                 ("tw1_bf16", C.c_void_p), ("tw2_bf16", C.c_void_p), ("workspace", C.c_void_p), ("loss", C.c_void_p),
-                ("max_batch", C.c_int32), ("reserved", C.c_int32)]
+                ("max_batch", C.c_int32), ("reserved", C.c_int32), ("dropout", C.c_float), ("update", C.c_int32), ("eval", C.c_int32),
+                ("reserved2", C.c_int32), ("dropout_seed", C.c_uint64), ("draw", C.c_uint64)]
 
 
 # flat parameter layout of the DQN / DDQN net (include/maze_b200.h MAZE_NET_*)

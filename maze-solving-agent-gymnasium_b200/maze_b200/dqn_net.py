@@ -6,10 +6,17 @@
     loss = net.train_step(*batch, gamma=0.9, lr=1e-4)              # double-Q target, MSE, clamp +-1, AdamW
     net.update_target()                                            # target_net.load_state_dict(source_net.state_dict())
 
+    DQNNet(device, dropout=0.2)                   # ddqn_agent.py as written: Dropout(0.2) in every forward
+    DQNNet(device, double_q=False)                # dqn_agent.py: y = r + gamma * max_a q_target(s', a)
+
 Everything runs in csrc/maze_net.cu through the C ABI (maze_dqn_forward / _backward / _adamw): tcgen05 GEMMs with
 TMA-staged bf16 operands for the conv (implicit GEMM) and the two big Linear layers, fp32 master weights.
 `state_dict()` / `load_state_dict()` speak the reference module's names (conv.0.weight, fc.0.weight, ...), so
-weights move between this class and the reference's `DQN` nn.Module unchanged.  Dropout is not applied.
+weights move between this class and the reference's `DQN` nn.Module unchanged.  Dropout (between the conv's
+LeakyReLU and its max-pool) is active in training mode (`train()`, the default: the reference never calls eval())
+and off after `eval()`.  Its masks come from a counter stream keyed by `dropout_seed` (include/maze_b200.h): every
+forward, features and backward call advances the net's draw counter, so two nets built alike and called alike
+produce identical bits.
 """
 from __future__ import annotations
 
@@ -35,7 +42,12 @@ def _views(flat: torch.Tensor):
 
 
 class DQNNet:
-    def __init__(self, device, max_batch: int = 8192, seed: int = 0, train: bool = True):
+    def __init__(self, device, max_batch: int = 8192, seed: int = 0, train: bool = True, dropout: float = 0.0, double_q: bool = True,
+                 dropout_seed: int | None = None):
+        """dropout: Dropout p in [0, 1) after the conv's LeakyReLU; double_q: the DDQN target (False: the DQN max target);
+        dropout_seed: key of the mask stream (default: `seed`)."""
+        if not 0.0 <= float(dropout) < 1.0:
+            raise ValueError(f"dropout must be in [0, 1), got {dropout}")
         self.device = torch.device(device)
         self.ctx = cabi.Context.for_device(self.device)
         self.max_batch = int(max_batch)
@@ -62,8 +74,41 @@ class DQNNet:
             params=self.params.data_ptr(), target=self.target.data_ptr(), grads=self.grads.data_ptr(), adam_m=self.adam_m.data_ptr(),
             adam_v=self.adam_v.data_ptr(), w1_bf16=self.w1_bf16.data_ptr(), w2_bf16=self.w2_bf16.data_ptr(),
             w1t_bf16=self.w1t_bf16.data_ptr(), w2t_bf16=self.w2t_bf16.data_ptr(), tw1_bf16=self.tw1_bf16.data_ptr(),
-            tw2_bf16=self.tw2_bf16.data_ptr(), workspace=ws_ptr, loss=self.loss.data_ptr(), max_batch=self.max_batch, reserved=0)
+            tw2_bf16=self.tw2_bf16.data_ptr(), workspace=ws_ptr, loss=self.loss.data_ptr(), max_batch=self.max_batch, reserved=0,
+            dropout=float(dropout), update=0 if double_q else 1, eval=0 if train else 1, reserved2=0,
+            dropout_seed=int(seed if dropout_seed is None else dropout_seed) & (2 ** 64 - 1), draw=0)
         self.reset_parameters(seed)
+
+    # ---- mode ---------------------------------------------------------------------------------------------------
+    @property
+    def dropout(self) -> float:
+        return float(self._c.dropout)
+
+    @property
+    def double_q(self) -> bool:
+        return self._c.update == 0
+
+    @property
+    def training(self) -> bool:
+        return self._c.eval == 0
+
+    def train(self, mode: bool = True):
+        """Training mode (dropout active), as nn.Module.train()."""
+        self._c.eval = 0 if mode else 1
+        return self
+
+    def eval(self):
+        """Evaluation mode (no dropout), as nn.Module.eval()."""
+        return self.train(False)
+
+    @property
+    def draw(self) -> int:
+        """The draw counter the next forward / features / backward call uses (then advances by one)."""
+        return int(self._c.draw)
+
+    def _next_draw(self):
+        """Each forward, features and backward call draws fresh dropout masks: the draw counter advances per call."""
+        self._c.draw = (self._c.draw + 1) & (2 ** 64 - 1)
 
     # ---- parameters -------------------------------------------------------------------------------------------
     def reset_parameters(self, seed: int = 0):
@@ -115,6 +160,7 @@ class DQNNet:
         rc = cabi.lib().maze_dqn_forward(self.ctx.handle, C.byref(self._c), int(which), cabi.ptr(vec), cabi.ptr(win), n, cabi.ptr(out),
                                          cabi.current_stream(self.device))
         self.ctx.check(rc, "maze_dqn_forward")
+        self._next_draw()
         return out
 
     def features(self, vec, win, which: int = 0, save_idx: bool = False):
@@ -124,6 +170,7 @@ class DQNNet:
         rc = cabi.lib().maze_dqn_features(self.ctx.handle, C.byref(self._c), int(which), cabi.ptr(vec), cabi.ptr(win), n, cabi.ptr(X),
                                           cabi.ptr(idx), cabi.current_stream(self.device))
         self.ctx.check(rc, "maze_dqn_features")
+        self._next_draw()
         return (X, idx) if save_idx else X
 
     def backward(self, vec, win, next_vec, next_win, action, reward, gamma: float, qsa_out: torch.Tensor | None = None,
@@ -136,6 +183,7 @@ class DQNNet:
                                           cabi.ptr(next_win), cabi.ptr(action), cabi.ptr(reward), n, float(gamma), cabi.ptr(qsa_out),
                                           ev, cabi.current_stream(self.device))
         self.ctx.check(rc, "maze_dqn_backward")
+        self._next_draw()
         return self.loss
 
     def profile(self, enable: bool):
